@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA hot path)
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed (.npy)
 
 A "step" is what pipelines/standard/train.lua:trainBatch does between its synchronisations:
 zeroGradParameters -> NETOBJ.ftrain (forward, ClassNLL, backward; models/basic_model.lua:56-62)
@@ -50,6 +51,26 @@ CONFIGS = {
 }
 CONFIG_METRIC = {"rmg34": METRIC, "rmg22": "R-MG-22 train images/sec", "prnmg30": "PR-NMG-30 train images/sec", "mg6": "MG-6 train images/sec",
                  "prnmg_mnist": "PR-NMG MNIST-cluttered train images/sec", "unmg": "U-MG MNIST-cluttered train images/sec"}
+
+
+# --dump-outputs: an array with more elements than this (16 MB in float32) is written as a sample, so that a dump of the
+# four arrays of a step stays under 64 MB
+DUMP_MAX_ELEMENTS = 1 << 22
+
+
+def dump_outputs(dirname, arrays):
+    """Write each tensor of `arrays` (name -> tensor) as DIR/<name>.npy in float32.  A larger array is replaced by the
+    elements of its flattened form at DUMP_MAX_ELEMENTS sorted indices drawn with a fixed seed: the same positions in
+    every run, so that the dumps of two builds compare element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        a = torch.as_tensor(t).detach().float()
+        if a.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(a.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(dirname, name + ".npy"), a.cpu().numpy())
 
 
 def peaks():
@@ -169,7 +190,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--bn-sync", action="store_true", help="cross-replica BatchNorm statistics (default: per replica, as the reference)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output, loss, parameters and parameter gradients of the last "
+                    "timed step as DIR/<name>.npy (float32; arrays above %d elements as a fixed seeded sample). Inputs and "
+                    "initial weights are seeded: two runs with the same arguments write the same values" % DUMP_MAX_ELEMENTS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computes; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -218,7 +246,7 @@ def main():
 
         def feval(_p):
             outputs, err = net.ftrain(x, t, model, criterion)
-            state["loss"] = err
+            state["outputs"], state["loss"] = outputs, err
             return err, grads
         net.btrain(params, feval, optimState)
 
@@ -250,6 +278,9 @@ def main():
     clocks = sampler.summary()
     ms = e0.elapsed_time(e1)
     launches = eng.ctx.launches() + cctx.launches() - l0
+    if args.dump_outputs and rank == 0:
+        # now, before the steps below overwrite the output buffers and move the parameters
+        dump_outputs(args.dump_outputs, {"output": state["outputs"], "loss": state["loss"], "parameters": params, "grad_parameters": grads})
     # Roofline of the convolution kernels: the timed region above runs WITHOUT the per-call event instrumentation (it costs
     # ~3 % of the step) and, with lanes, overlaps kernels of different scales, so a kernel's own duration cannot be read
     # there.  It is taken from extra steps of the SERIAL plan (one stream, kernels back to back -- what the ncu launch

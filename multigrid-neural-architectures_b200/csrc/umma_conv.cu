@@ -1931,7 +1931,7 @@ static int persist_tile_rows(const mg_conv_desc* d, int Nimg, bool any_up) {
   (void)Nimg;
   return R;
 }
-static bool persist_plan(const mg_ctx* ctx, const mg_conv_desc* d, const Geometry& g, int Nimg, int algo, PersistPlan* pl) {
+static bool persist_plan(const mg_ctx* ctx, const mg_conv_desc* d, const Geometry& g, int Nimg, int algo, bool stats, PersistPlan* pl) {
   static int on = -1, min_tiles_per_sm = -1;
   if (on < 0) { const char* e = getenv("MGCONV_PERSIST"); on = e ? atoi(e) : 1; }
   if (min_tiles_per_sm < 0) { const char* e = getenv("MGCONV_PERSIST_MIN_TILES"); min_tiles_per_sm = e ? atoi(e) : 4; }
@@ -1947,10 +1947,13 @@ static bool persist_plan(const mg_ctx* ctx, const mg_conv_desc* d, const Geometr
   bool any_up = false;
   for (int s = 0; s < d->n_seg; ++s) any_up = any_up || d->seg_mode[s] == MG_SEG_UP;
   // row-aligned tiles: always for CTA pairs (same tile offset in both CTAs); for the single-CTA kernel only on request -- its
-  // ring stays two tiles short either way and 12 % more tiles cost more than the smaller halo saves (measured: 125 -> 133 us)
+  // ring stays two tiles short either way and 12 % more tiles cost more than the smaller halo saves (measured: 125 -> 133 us).
+  // Never when the epilogue reduces BatchNorm statistics: each warp sums its 32 slots in fp32 before the exact fixed-point total,
+  // and only 128-slot tiles give every warp the same 32 slots in every variant; with R * Wp-slot tiles the statistics (and all
+  // that follows them) would depend on which variant the autotuner timed fastest.
   static int aligned_single = -1;
   if (aligned_single < 0) { const char* e = getenv("MGCONV_PERSIST_ALIGNED"); aligned_single = e ? atoi(e) : 0; }
-  const int R = (pair || aligned_single) ? persist_tile_rows(d, Nimg, any_up && g.n_chunks > 0) : 0;
+  const int R = ((pair || aligned_single) && !stats) ? persist_tile_rows(d, Nimg, any_up && g.n_chunks > 0) : 0;
   if (R) hp.halo_bytes = mg_round_up(((R + 2) * hp.Wp + 2) * 128, 1024);
   const int64_t m_tiles = R ? mg_cdiv((int64_t)Nimg * (d->H + 1), R) : mg_cdiv((int64_t)Nimg * (d->H + 1) * hp.Wp, BM);
   if (!forced && m_tiles < (int64_t)min_tiles_per_sm * ctx->num_sms) return false;
@@ -2185,7 +2188,7 @@ int umma_conv_forward(mg_ctx* ctx, const mg_conv_desc* d, const void* wpack, con
     const bool fused_stats = bn_sums && fused_stats_on();
     if (fused_stats) { hp.stats = bn_sums; hp.c_stats = d->Cout; }
     PersistPlan pl;
-    rc = persist_plan(ctx, d, g, hp.Nimg, d->algo_fwd, &pl) ? launch_halo_persistent(ctx, hp, pl, d->seg) : launch_halo(ctx, hp, g, d->algo_fwd, d->seg);
+    rc = persist_plan(ctx, d, g, hp.Nimg, d->algo_fwd, hp.stats != nullptr, &pl) ? launch_halo_persistent(ctx, hp, pl, d->seg) : launch_halo(ctx, hp, g, d->algo_fwd, d->seg);
     if (rc) return rc;
     if (bn_sums && !fused_stats) return mg_bn_stats(ctx, y, bn_sums);
     return MG_OK;
@@ -2224,7 +2227,7 @@ int umma_conv_backward_data(mg_ctx* ctx, const mg_conv_desc* d, const void* wpac
     hp.wpack = (const uint8_t*)wpack_t; hp.bias = nullptr;
     hp.y = (__nv_bfloat16*)dcat->data; hp.y_pitch = dcat->Cp; hp.c_valid = dcat->Cp;
     PersistPlan pl;
-    return persist_plan(ctx, d, g, hp.Nimg, d->algo_bwd_data, &pl) ? launch_halo_persistent(ctx, hp, pl, gr) : launch_halo(ctx, hp, g, d->algo_bwd_data, gr);
+    return persist_plan(ctx, d, g, hp.Nimg, d->algo_bwd_data, false, &pl) ? launch_halo_persistent(ctx, hp, pl, gr) : launch_halo(ctx, hp, g, d->algo_bwd_data, gr);
   }
   UParams p;
   memset(&p, 0, sizeof(p));

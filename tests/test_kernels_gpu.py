@@ -493,6 +493,40 @@ def test_persistent_weight_resident_kernel_block1_shape():
     ctx.close()
 
 
+def test_every_kernel_variant_computes_the_same_bits():
+    """The variant of a 3x3 layer is chosen by timing (Engine autotune), so the choice must not change a bit: forward output, its
+    fused BatchNorm sums and dgrad of every MG_ALGO_* equal the heuristic's.  At 56x56 and 28x28 the persistent CTA-pair kernel
+    would use row-aligned tiles (R * (W + 1) slots), which group the slots of the fp32 partial sums differently"""
+    ctx = ffi.Context(0, torch.cuda.current_stream().cuda_stream, ffi.MG_BF16)
+    for (N, H, cs, Cout) in [(32, 56, (64, 32), 64), (112, 28, (64, 32, 16), 32)]:
+        grids = [Grid(ffi.MG_BF16, N, cs[0], H, H)] + [Grid(ffi.MG_BF16, N, c, H, H) for c in cs[1:-1]] + [Grid(ffi.MG_BF16, N, cs[-1], H // 2, H // 2)]
+        modes = [MG_SEG_SAME] * (len(cs) - 1) + [MG_SEG_UP]
+        for g_ in grids:
+            g_.t[..., :g_.C].normal_()
+        d = conv_desc(grids, modes, 3, 1, 1, Cout, H, H)
+        w = (torch.randn(Cout, sum(cs), 3, 3, device="cuda") * 0.05).to(torch.bfloat16).float()
+        b = (torch.randn(Cout, device="cuda") * 0.1).to(torch.bfloat16).float()
+        wp = torch.zeros(ffi.lib.mg_conv_packed_bytes(C.byref(d), 0), dtype=torch.uint8, device="cuda")
+        wpt = torch.zeros(ffi.lib.mg_conv_packed_bytes(C.byref(d), 1), dtype=torch.uint8, device="cuda")
+        ctx.call("mg_conv_pack_weights", C.byref(d), ptr(w), ptr(wp), 0)
+        ctx.call("mg_conv_pack_weights", C.byref(d), ptr(w), ptr(wpt), 1)
+        gg = Grid(ffi.MG_BF16, N, Cout, H, H)
+        gg.t[..., :Cout].normal_()
+        cp = sum(x.Cp for x in grids)
+        ref = None
+        for algo in range(ffi.MG_ALGO_RESIDENT_PAIR + 1):
+            d.algo_fwd = d.algo_bwd_data = algo
+            gy, sums, dcat = Grid(ffi.MG_BF16, N, Cout, H, H), new_sums(2 * Cout), Grid(ffi.MG_BF16, N, cp, H, H, Cp=cp)
+            ctx.call("mg_conv_forward", C.byref(d), ptr(w), ptr(wp), ptr(b), C.byref(gy.g()), ptr(sums))
+            ctx.call("mg_conv_backward_data", C.byref(d), ptr(w), ptr(wpt), C.byref(gg.g()), C.byref(dcat.g()))
+            torch.cuda.synchronize()
+            got = (gy.t, sums, dcat.t)
+            ref = ref or got
+            for name, a, r in zip(("output", "BatchNorm sums", "dgrad"), got, ref):
+                assert torch.equal(a, r), (H, algo, name)
+    ctx.close()
+
+
 FULL_SHAPES = [  # R-MG-34 layers at the BASELINE batch (256 per GPU): (H, [(C, mode)], Cout)
     (56, [(64, "s"), (32, "u")], 64),                # block 1, finest grid (rnmg.lua:250)
     (28, [(128, "s"), (64, "s"), (32, "u")], 64),    # block 2, middle grid: pooled finer | same | up-sampled coarser
