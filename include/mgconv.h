@@ -245,6 +245,29 @@ int mg_upconv2x2_forward(mg_ctx* ctx, const mg_grid* x, const float* w, const fl
 int mg_upconv2x2_backward(mg_ctx* ctx, const mg_grid* x, const float* w, const mg_grid* g, mg_grid* dx,
                           float* dw, float* dbias, float gscale);
 
+/* nn.Dropout(p) in training mode, Torch7's default (v2) form: y = x * mask * s, dx = dy * mask * s, mask in {0,1} with
+ * P(keep) = 1 - p, s = fp32(1 / (1 - p)).  models/cifar/pnmg.lua:25-27 puts one in front of every convolution of blocks 2-5
+ * when -isDropout.  The mask is counter based and never stored: element i, its NHWC index over the logical channels (pad
+ * channels excluded), is kept iff word (i & 3) of Philox4x32-10(counter = (i >> 2, op, (uint32) *step, rank), key = (seed lo,
+ * seed hi)) is >= t = min(2^32 - 1, floor(p * 2^32)).  *step is a device counter that mg_dropout_advance increments once per
+ * training forward, so a captured CUDA graph draws a fresh mask on every replay; backward regenerates the forward's mask
+ * from the same (seed, op, step, rank).  Every call rejects p < 0 and p >= 1. */
+typedef struct {
+  float p;               /* drop probability */
+  uint32_t op;           /* ordinal of the dropout in the plan: masks of different dropouts are independent */
+  uint32_t rank;         /* data-parallel rank (0 on one device): shards do not share masks */
+  uint64_t seed;         /* Philox key */
+  const uint64_t* step;  /* device */
+} mg_dropout;
+/* out = dropout(cat_C[ seg_0 | seg_1 | ... ]) as one tensor (pad channels written as zero).  seg_mode: MG_SEG_SAME (read at the
+ * output resolution, pooled companions included) or MG_SEG_UP (coarser grid read at (y/2, x/2)); every mask element of an
+ * up-sampled pixel is drawn independently, which is why the concatenation is materialised instead of gathered by the conv. */
+int mg_dropout_forward(mg_ctx* ctx, const mg_dropout* dp, int32_t n_seg, const mg_grid* seg, const int32_t* seg_mode, mg_grid* out);
+/* in place: g = g * mask * s (pad channels untouched) */
+int mg_dropout_backward(mg_ctx* ctx, const mg_dropout* dp, mg_grid* g);
+/* ++*step on the context stream */
+int mg_dropout_advance(mg_ctx* ctx, uint64_t* step);
+
 /* ---- backward ------------------------------------------------------------------------- */
 /* Sum of all consumers' gradient contributions into tensor x (ConcatTable backward sums
  * its branches), routed through pool argmax / upsample block-sum, times the ReLU mask of x

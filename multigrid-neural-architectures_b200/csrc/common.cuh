@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+#include <curand_philox4x32_x.h>
 #include "../../include/mgconv.h"
 
 #define MG_MAX_LANES 4
@@ -158,6 +159,58 @@ static inline GridV<T> make_view(const mg_grid& g) {
 }
 
 static inline size_t mg_elt_size(int dtype) { return dtype == MG_BF16 ? 2 : 4; }
+
+// ---- counter-based dropout mask (mg_dropout, see mgconv.h) ------------------------------------------------------
+// element i (NHWC index over the logical channels) is kept iff word i & 3 of Philox4x32-10((i >> 2, op, step, rank), seed) >= t
+struct DropK {
+  uint32_t key_lo, key_hi, op, rank, t;
+  float s;                 // fp32(1 / (1 - p))
+  const uint64_t* step;
+};
+
+// bit e of the result: element i0 + e is kept (n <= 8 consecutive elements, at most three Philox calls)
+__device__ __forceinline__ uint32_t drop_keep_bits(uint64_t i0, int n, const DropK& k) {
+  const uint32_t step = (uint32_t)*k.step;
+  uint32_t bits = 0;
+  for (uint64_t g = i0 >> 2; g <= (i0 + n - 1) >> 2; ++g) {
+    const uint4 u = curand_Philox4x32_10(make_uint4((uint32_t)g, k.op, step, k.rank), make_uint2(k.key_lo, k.key_hi));
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int64_t e = (int64_t)(4 * g + j) - (int64_t)i0;
+      if (e >= 0 && e < n && w[j] >= k.t) bits |= 1u << e;
+    }
+  }
+  return bits;
+}
+
+// the source segments of mg_dropout_forward: output channel c belongs to segment s when off[s] <= c < off[s + 1]
+template <typename T>
+struct DropSegs {
+  int n;
+  GridV<T> g[MG_MAX_SEG];
+  int up[MG_MAX_SEG];      // MG_SEG_UP: read at (y / 2, x / 2)
+  int off[MG_MAX_SEG + 1];
+};
+template <typename T>
+static inline DropSegs<T> make_drop_segs(int n, const mg_grid* seg, const int32_t* mode) {
+  DropSegs<T> d;
+  memset(&d, 0, sizeof(d));
+  d.n = n;
+  for (int s = 0; s < n; ++s) {
+    d.g[s] = make_view<T>(seg[s]);
+    d.up[s] = mode[s] == MG_SEG_UP;
+    d.off[s + 1] = d.off[s] + seg[s].C;
+  }
+  return d;
+}
+// value of output channel c at (n, y, x) of the concatenation
+template <typename T>
+__device__ __forceinline__ float drop_gather(const DropSegs<T>& d, int n, int y, int x, int c) {
+  int s = 0;
+  while (s + 1 < d.n && c >= d.off[s + 1]) ++s;
+  return d.up[s] ? d.g[s].at(n, y >> 1, x >> 1, c - d.off[s]) : d.g[s].at(n, y, x, c - d.off[s]);
+}
 
 // dispatch on the context dtype
 #define MG_DISPATCH(ctx, ...)                          \

@@ -20,6 +20,8 @@ bool bf16_bn_relu_pool3(mg_ctx*, const mg_grid* z, const mg_bn_fused* bn, mg_gri
 bool bf16_import_nchw(mg_ctx*, const float* src, mg_grid* dst);
 bool bf16_avgpool(mg_ctx*, const mg_grid* in, int r, mg_grid* out);
 bool bf16_pool2(mg_ctx*, const mg_grid* in, mg_grid* out, int c_off);
+bool bf16_dropout_forward(mg_ctx*, const DropK& k, int n_seg, const mg_grid* seg, const int32_t* mode, mg_grid* out);
+bool bf16_dropout_backward(mg_ctx*, const DropK& k, mg_grid* g);
 
 namespace {
 
@@ -447,7 +449,53 @@ __global__ void sgd_kernel(float* __restrict__ w, const float* __restrict__ g, f
   w[i] = fmaf(-lr, vi, w[i]);
 }
 
+// ---------------------------------------------------------------- dropout -----------
+// one thread per (pixel, 4 channels of the pitch); the logical elements of a quad span at most two Philox calls
+template <typename T>
+__global__ void dropout_fwd_kernel(DropSegs<T> d, DropK k, T* __restrict__ out, int N, int H, int W, int C, int Cp) {
+  const int64_t i = (int64_t)blockIdx.x * EB + threadIdx.x;
+  const int Q = Cp / 4;
+  if (i >= (int64_t)N * H * W * Q) return;
+  const int q = i % Q; const int64_t pix = i / Q;
+  const int x = pix % W; const int64_t r = pix / W; const int y = r % H; const int n = r / H;
+  const int c0 = q * 4, nl = min(4, C - c0);   // logical channels of the quad (none: pad only)
+  const uint32_t keep = nl > 0 ? drop_keep_bits((uint64_t)pix * C + c0, nl, k) : 0u;
+  for (int e = 0; e < 4; ++e) {
+    float v = 0.f;
+    if (e < nl && (keep >> e & 1u)) v = drop_gather(d, n, y, x, c0 + e) * k.s;
+    mg_st(out + pix * Cp + c0 + e, v);
+  }
+}
+
+template <typename T>
+__global__ void dropout_bwd_kernel(DropK k, T* __restrict__ g, int64_t P, int C, int Cp) {
+  const int64_t i = (int64_t)blockIdx.x * EB + threadIdx.x;
+  const int Q = Cp / 4;
+  if (i >= P * Q) return;
+  const int q = i % Q; const int64_t pix = i / Q;
+  const int c0 = q * 4, nl = min(4, C - c0);
+  if (nl <= 0) return;
+  const uint32_t keep = drop_keep_bits((uint64_t)pix * C + c0, nl, k);
+  for (int e = 0; e < nl; ++e) {
+    T* p = g + pix * Cp + c0 + e;
+    mg_st(p, (keep >> e & 1u) ? mg_ld(p) * k.s : 0.f);
+  }
+}
+
+__global__ void dropout_advance_kernel(uint64_t* step) { ++*step; }
+
 }  // namespace
+
+// mask parameters of a dropout call; rejects p outside [0, 1)
+static int drop_key(mg_ctx* ctx, const mg_dropout* dp, DropK* k) {
+  MG_REQUIRE(ctx, dp->p >= 0.f && dp->p < 1.f, MG_ERR_INVALID_ARG, "dropout: p = %g is outside [0, 1)", (double)dp->p);
+  MG_REQUIRE(ctx, dp->step != nullptr, MG_ERR_INVALID_ARG, "dropout: null step counter");
+  k->key_lo = (uint32_t)dp->seed; k->key_hi = (uint32_t)(dp->seed >> 32);
+  k->op = dp->op; k->rank = dp->rank; k->step = dp->step;
+  k->t = (uint32_t)std::min(floor((double)dp->p * 4294967296.0), 4294967295.0);
+  k->s = (float)(1.0 / (1.0 - (double)dp->p));
+  return MG_OK;
+}
 
 #define GRID1(total) (unsigned)mg_cdiv((int64_t)(total), EB)
 
@@ -573,6 +621,51 @@ int mg_copy_channels(mg_ctx* ctx, const mg_grid* in, mg_grid* out, int32_t c_off
   MG_REQUIRE(ctx, out->H == in->H && out->W == in->W && out->N == in->N && c_offset + in->C <= out->Cp, MG_ERR_SHAPE, "copy_channels: shape");
   int64_t total = (int64_t)in->N * in->H * in->W * in->C;
   MG_DISPATCH(ctx, copy_channels_kernel<T><<<GRID1(total), EB, 0, ctx->stream>>>(make_view<T>(*in), (T*)out->data, out->Cp, c_offset););
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
+int mg_dropout_forward(mg_ctx* ctx, const mg_dropout* dp, int32_t n_seg, const mg_grid* seg, const int32_t* seg_mode, mg_grid* out) {
+  if (!ctx || !dp || !seg || !seg_mode || !out || !out->data || n_seg < 1 || n_seg > MG_MAX_SEG) return MG_ERR_INVALID_ARG;
+  DropK k;
+  int rc = drop_key(ctx, dp, &k);
+  if (rc) return rc;
+  int C = 0;
+  for (int s = 0; s < n_seg; ++s) {
+    const mg_grid& g = seg[s];
+    MG_REQUIRE(ctx, seg_mode[s] == MG_SEG_SAME || seg_mode[s] == MG_SEG_UP, MG_ERR_INVALID_ARG, "dropout_forward: segment %d mode %d", s, seg_mode[s]);
+    const int f = seg_mode[s] == MG_SEG_UP ? 2 : 1;
+    MG_REQUIRE(ctx, g.data && g.N == out->N && f * g.H == out->H && f * g.W == out->W && g.C <= g.Cp, MG_ERR_SHAPE,
+               "dropout_forward: segment %d (mode %d) is %dx%d, output %dx%d", s, seg_mode[s], g.H, g.W, out->H, out->W);
+    C += g.C;
+  }
+  MG_REQUIRE(ctx, C == out->C && out->Cp >= out->C && out->Cp % 8 == 0, MG_ERR_SHAPE, "dropout_forward: %d channels into C %d Cp %d", C, out->C, out->Cp);
+  const int64_t P = (int64_t)out->N * out->H * out->W;
+  MG_REQUIRE(ctx, P * C < ((int64_t)1 << 34), MG_ERR_SHAPE, "dropout_forward: %lld elements exceed the 2^34 of the Philox counter", (long long)(P * C));
+  if (ctx->dtype == MG_BF16 && bf16_dropout_forward(ctx, k, n_seg, seg, seg_mode, out)) { MG_CHECK_LAUNCH(ctx); return MG_OK; }
+  MG_DISPATCH(ctx, dropout_fwd_kernel<T><<<GRID1(P * (out->Cp / 4)), EB, 0, ctx->stream>>>(make_drop_segs<T>(n_seg, seg, seg_mode), k, (T*)out->data,
+                                                                                        out->N, out->H, out->W, out->C, out->Cp););
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
+int mg_dropout_backward(mg_ctx* ctx, const mg_dropout* dp, mg_grid* g) {
+  if (!ctx || !dp || !g || !g->data) return MG_ERR_INVALID_ARG;
+  DropK k;
+  int rc = drop_key(ctx, dp, &k);
+  if (rc) return rc;
+  MG_REQUIRE(ctx, g->Cp >= g->C && g->Cp % 8 == 0, MG_ERR_SHAPE, "dropout_backward: C %d Cp %d", g->C, g->Cp);
+  const int64_t P = (int64_t)g->N * g->H * g->W;
+  MG_REQUIRE(ctx, P * g->C < ((int64_t)1 << 34), MG_ERR_SHAPE, "dropout_backward: %lld elements exceed the 2^34 of the Philox counter", (long long)(P * g->C));
+  if (ctx->dtype == MG_BF16 && bf16_dropout_backward(ctx, k, g)) { MG_CHECK_LAUNCH(ctx); return MG_OK; }
+  MG_DISPATCH(ctx, dropout_bwd_kernel<T><<<GRID1(P * (g->Cp / 4)), EB, 0, ctx->stream>>>(k, (T*)g->data, P, g->C, g->Cp););
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
+int mg_dropout_advance(mg_ctx* ctx, uint64_t* step) {
+  if (!ctx || !step) return MG_ERR_INVALID_ARG;
+  dropout_advance_kernel<<<1, 1, 0, ctx->stream>>>(step);
   MG_CHECK_LAUNCH(ctx);
   return MG_OK;
 }

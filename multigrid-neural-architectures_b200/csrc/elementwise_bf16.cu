@@ -864,6 +864,58 @@ __global__ void __launch_bounds__(256) im2col_bf16_kernel(const bf16* __restrict
   *reinterpret_cast<uint4*>(col + i * 8) = make_uint4(w[0], w[1], w[2], w[3]);
 }
 
+// ---------------------------------------------------------------- dropout ----------
+// nn.Dropout in training mode (mgconv.h: mg_dropout).  One thread per (pixel, 8 channels of the pitch), one 16-byte store.  A
+// vector whose 8 channels lie in one segment, starting at a multiple of 8 of its channels, is read with one 16-byte load; any
+// other (segments whose C is not a multiple of 8) element by element.  Same expressions as dropout_fwd_kernel (elementwise.cu).
+__global__ void __launch_bounds__(256) dropout_fwd_bf16_kernel(const __grid_constant__ DropSegs<bf16> d, const DropK k, bf16* __restrict__ out,
+                                                               int N, int H, int W, int C, int V) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (int64_t)N * H * W * V) return;
+  int n, y, x, vc;
+  split4(i, H, W, V, n, y, x, vc);
+  const int64_t pix = ((int64_t)n * H + y) * W + x;
+  const int c0 = vc * 8, nl = min(8, C - c0);
+  V8 o;
+#pragma unroll
+  for (int e = 0; e < 8; ++e) o.v[e] = 0.f;
+  if (nl > 0) {
+    const uint32_t keep = drop_keep_bits((uint64_t)pix * C + c0, nl, k);
+    int s = 0;
+    while (s + 1 < d.n && c0 >= d.off[s + 1]) ++s;
+    const GridV<bf16>& G = d.g[s];
+    const int lc = c0 - d.off[s];
+    if (nl == 8 && c0 + 8 <= d.off[s + 1] && lc % 8 == 0 && !G.scale) {
+      const int yy = d.up[s] ? y >> 1 : y, xx = d.up[s] ? x >> 1 : x;
+      const V8 v = ld8(G.data + (((int64_t)n * G.H + yy) * G.W + xx) * G.Cp + lc);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) o.v[e] = (keep >> e & 1u) ? v.v[e] * k.s : 0.f;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 8; ++e)
+        if (e < nl && (keep >> e & 1u)) o.v[e] = drop_gather(d, n, y, x, c0 + e) * k.s;
+    }
+  }
+  *reinterpret_cast<uint4*>(out + i * 8) = pack8(o);
+}
+
+// in place g = g * mask * s, 8 channels (one 16-byte load and store) per thread; pad channels are stored back unchanged
+__global__ void __launch_bounds__(256) dropout_bwd_bf16_kernel(const DropK k, bf16* __restrict__ g, int64_t P, int C, int V) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P * V) return;
+  int64_t pix; int vc;
+  if (i < ((int64_t)1 << 32)) { const uint32_t q = (uint32_t)i / (uint32_t)V; pix = q; vc = (int)((uint32_t)i - q * (uint32_t)V); }
+  else { pix = i / V; vc = (int)(i - pix * V); }
+  const int c0 = vc * 8, nl = min(8, C - c0);
+  if (nl <= 0) return;
+  const uint32_t keep = drop_keep_bits((uint64_t)pix * C + c0, nl, k);
+  V8 v = ld8(g + i * 8);
+#pragma unroll
+  for (int e = 0; e < 8; ++e)
+    if (e < nl) v.v[e] = (keep >> e & 1u) ? v.v[e] * k.s : 0.f;
+  *reinterpret_cast<uint4*>(g + i * 8) = pack8(v);
+}
+
 static inline unsigned grid_for(int64_t threads) { return (unsigned)mg_cdiv(threads, 256); }
 // persistent-style grid for the reducing kernels: a few CTAs per SM, each thread loops
 static inline unsigned reduce_grid(const mg_ctx* ctx, int64_t items, int per_sm = 4) {
@@ -1032,6 +1084,23 @@ bool bf16_avgpool(mg_ctx* ctx, const mg_grid* in, int r, mg_grid* out) {
   const int64_t total = (int64_t)in->N * out->H * out->W * (in->Cp / 8);
   pool_vec_kernel<false><<<grid_for(total), 256, 0, ctx->stream>>>((const bf16*)in->data, in->H, in->W, in->Cp, in->C, r, (bf16*)out->data,
                                                                    out->H, out->W, out->Cp, 0, in->N);
+  return true;
+}
+
+bool bf16_dropout_forward(mg_ctx* ctx, const DropK& k, int n_seg, const mg_grid* seg, const int32_t* mode, mg_grid* out) {
+  for (int s = 0; s < n_seg; ++s)
+    if (seg[s].Cp % 8) return false;
+  const int V = out->Cp / 8;
+  const int64_t total = (int64_t)out->N * out->H * out->W * V;
+  dropout_fwd_bf16_kernel<<<grid_for(total), 256, 0, ctx->stream>>>(make_drop_segs<bf16>(n_seg, seg, mode), k, (bf16*)out->data, out->N, out->H,
+                                                                    out->W, out->C, V);
+  return true;
+}
+
+bool bf16_dropout_backward(mg_ctx* ctx, const DropK& k, mg_grid* g) {
+  const int V = g->Cp / 8;
+  const int64_t P = (int64_t)g->N * g->H * g->W;
+  dropout_bwd_bf16_kernel<<<grid_for(P * V), 256, 0, ctx->stream>>>(k, (bf16*)g->data, P, g->C, V);
   return true;
 }
 

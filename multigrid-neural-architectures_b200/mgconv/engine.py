@@ -35,10 +35,16 @@ def _flatten(x):
     return [x]
 
 
-def engine_key(input):
+def engine_key(input, dropouts=()):
+    """plans are kept per input shape and device; a model with an active nn.Dropout (`dropouts`: its nn.Dropout modules) also
+    gets one plan per mode (training plans hold the dropout ops, evaluation plans are those of the same model without them)"""
     ts = _flatten(input)
-    return (tuple(input.shape) if isinstance(input, torch.Tensor) else tuple(tuple(t.shape) for t in ts),
-            ts[0].device.index)
+    key = (tuple(input.shape) if isinstance(input, torch.Tensor) else tuple(tuple(t.shape) for t in ts),
+           ts[0].device.index)
+    active = [m for m in dropouts if m.p > 0]
+    if active:
+        key += (any(m.train for m in active),)
+    return key
 
 
 class Engine:
@@ -50,7 +56,7 @@ class Engine:
                                   "call model:cuda() and move the inputs with put2GPU first")
         self.model = model
         self.device = inputs[0].device
-        self.key = engine_key(input)
+        self.key = engine_key(input, model.findModules("nn.Dropout"))
         precision = getattr(model, "precision", os.environ.get("MGCONV_PRECISION", "bf16"))
         self.dtype, self.elt = _PRECISION[precision]
         self.ctx = ffi.Context(self.device.index, torch.cuda.current_stream(self.device).cuda_stream, self.dtype)
@@ -83,6 +89,12 @@ class Engine:
                                    bool(getattr(model, "needInputGrad", False)))
         self.out_struct = self._wrap_outputs(out, b)
         self.plan = b
+        # Philox key of the plan's dropout masks, drawn from torch's default generator (torch.manual_seed fixes every mask)
+        self.dropout_seed = 0
+        if b.drops:
+            lo, hi = torch.randint(0, 1 << 32, (2,), dtype=torch.int64).tolist()
+            self.dropout_seed = lo | hi << 32
+        self._dropout_rank = 0
         self.input_ops = [o for o in b.ops if isinstance(o, ops.InputOp)]
         self.conv_ops = [o for o in b.ops if isinstance(o, ops.ConvOp)]
         ops.fuse_stem_pool3(b.ops, self)
@@ -136,6 +148,17 @@ class Engine:
     def set_bn_sync(self, nranks):
         """0 = per-replica BatchNorm statistics (the reference's DataParallelTable), N = statistics over N equal shards"""
         self.bn_sync = int(nranks)
+
+    @property
+    def dropout_rank(self):
+        """data-parallel rank: a word of the dropout mask counter, so that shards draw different masks"""
+        return self._dropout_rank
+
+    @dropout_rank.setter
+    def dropout_rank(self, rank):
+        self._dropout_rank = int(rank)
+        for o in self.plan.drops:
+            o.dp.rank = self._dropout_rank
 
     def _use_lanes(self):
         # cross-replica BatchNorm issues NCCL calls from inside the chains: those must stay on one stream

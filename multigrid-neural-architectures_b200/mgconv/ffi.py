@@ -60,6 +60,10 @@ class mg_bn_fused(C.Structure):
                 ("training", C.c_int32), ("save_mean", C.c_void_p), ("save_invstd", C.c_void_p)]
 
 
+class mg_dropout(C.Structure):
+    _fields_ = [("p", C.c_float), ("op", C.c_uint32), ("rank", C.c_uint32), ("seed", C.c_uint64), ("step", C.c_void_p)]
+
+
 def _load():
     if not os.path.exists(LIB_PATH):
         raise MGError(
@@ -113,6 +117,9 @@ SIGNATURES = {
     "mg_global_avgpool_backward": (_I, [_P, _G, _G]),
     "mg_upconv2x2_forward": (_I, [_P, _G, _P, _P, _G, _P]),
     "mg_upconv2x2_backward": (_I, [_P, _G, _P, _G, _G, _P, _P, _F]),
+    "mg_dropout_forward": (_I, [_P, C.POINTER(mg_dropout), C.c_int32, _G, C.POINTER(C.c_int32), _G]),
+    "mg_dropout_backward": (_I, [_P, C.POINTER(mg_dropout), _G]),
+    "mg_dropout_advance": (_I, [_P, _P]),
     "mg_grad_combine": (_I, [_P, _G, _I, _G, C.c_int32, C.POINTER(mg_grad_src), _G, _P]),
     "mg_bn_backward": (_I, [_P, _G, _G, _G, _P, _I64, _P, _P, _P, _P, _P, _F, _P, _P]),
     "mg_conv_backward_data": (_I, [_P, _D, _P, _P, _G, _G]),

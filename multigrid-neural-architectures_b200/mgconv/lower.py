@@ -7,6 +7,8 @@ Values flowing through the trace:
   NodeVal  output of a convolution whose epilogue (BN, ReLU, shortcut add, ReLU) is still being
            collected; `seal` turns it into a TVal by emitting the apply pass
   PadVal   nn.Padding(1, p, 3) of a value (only meaningful as the shortcut operand of CAddTable)
+  DropVal  nn.Dropout(p) of a value in training mode -- materialised by a DropOp (the dropped concatenation of the value's
+           segments) the first time a convolution or shortcut consumes it
   OutVal   fp32 network output at the Torch boundary (log-probabilities / probabilities)
 
 max-pool 2x2/ceil of a tensor is its *pooled companion*: written by the producer's apply pass
@@ -81,6 +83,15 @@ class PadVal(Val):
     W = property(lambda s: s.src.W)
 
 
+class DropVal(Val):
+    def __init__(self, src, p):
+        self.src, self.p = src, p
+        self.out = None      # TVal once materialised
+    C = property(lambda s: s.src.C)
+    H = property(lambda s: s.src.H)
+    W = property(lambda s: s.src.W)
+
+
 class OutVal(Val):
     def __init__(self, op, shape):
         self.op, self.shape = op, shape
@@ -93,6 +104,8 @@ class Builder:
         self.N = N
         self.tensors = []
         self.ops = []
+        self.drops = []      # DropOps in plan order: their index is the `op` word of the mask counter
+        self.drop_step = None
 
     # ---- tensors ------------------------------------------------------------------------
     def new_tensor(self, C, H, W, name, needs_grad=True):
@@ -142,6 +155,8 @@ class Builder:
         v = self.resolve(v)
         if isinstance(v, TVal):
             return v
+        if isinstance(v, DropVal):
+            return self.drop(v)
         if isinstance(v, CatVal):
             segs = self.segments(v)
             if any(m != MG_SEG_SAME for _, m in segs):
@@ -157,6 +172,8 @@ class Builder:
             return [(v.spec, MG_SEG_SAME)]
         if isinstance(v, UpVal):
             return [(v.src.spec, MG_SEG_UP)]
+        if isinstance(v, DropVal):
+            return [(self.drop(v).spec, MG_SEG_SAME)]
         if isinstance(v, CatVal):
             out = []
             for p in v.parts:
@@ -164,7 +181,27 @@ class Builder:
             return out
         raise NotImplementedError(f"{type(v).__name__} cannot feed a convolution")
 
+    def drop(self, v):
+        """the dropped concatenation of v's segments as one tensor (one mask shared by every consumer, like the output of
+        a Torch7 nn.Dropout); the plan's step counter is advanced right before its first DropOp"""
+        if v.out is None:
+            segs = self.segments(v.src)
+            if len(segs) > MG_MAX_SEG:
+                raise NotImplementedError(f"nn.Dropout of {len(segs)} segments > MG_MAX_SEG")
+            if self.drop_step is None:
+                self.drop_step = self.emit(O.DropStepOp())
+            out = self.new_tensor(v.C, v.H, v.W, f"drop{len(self.drops)}", needs_grad=any(t.needs_grad for t, _ in segs))
+            self.drops.append(self.emit(O.DropOp(segs, v.p, len(self.drops), self.drop_step, out)))
+            v.out = TVal(out)
+        return v.out
+
     # ---- ops called by the modules ---------------------------------------------------------
+    def dropout(self, v, p):
+        v = self.resolve(v)
+        if isinstance(v, (DropVal, PadVal, OutVal)):
+            raise NotImplementedError(f"nn.Dropout of {type(v).__name__}: not a pattern of the builders")
+        return DropVal(v, p)
+
     def cat(self, parts):
         parts = [self.resolve(p) for p in parts]
         return parts[0] if len(parts) == 1 else CatVal(parts)

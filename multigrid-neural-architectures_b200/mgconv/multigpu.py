@@ -182,7 +182,8 @@ class DataParallel:
         return self._shards[local_B]
 
     def _attach(self, eng, input):
-        """bind a (new or cached) engine to this wrapper BEFORE it runs: bucket triggers, communicator, shard weights"""
+        """bind a (new or cached) engine to this wrapper BEFORE it runs: dropout rank, bucket triggers, communicator, shard weights"""
+        eng.dropout_rank = self.rank
         if self.world == 1:
             return
         ts = input

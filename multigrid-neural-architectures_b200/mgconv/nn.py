@@ -32,6 +32,7 @@ class Module:
         self.output = None
         self.gradInput = None
         self._engine = None
+        self._dropouts = None
 
     # ---- graph walking ----------------------------------------------------------------
     def children(self):
@@ -119,6 +120,7 @@ class Module:
         for m in self.listModules():
             m._engine = None
             m._engines = None
+            m._dropouts = None
             m.output = None
             m.gradInput = None
         return self
@@ -127,7 +129,9 @@ class Module:
     def _get_engine(self, input):
         from .engine import Engine
         from .engine import engine_key
-        key = engine_key(input)
+        if self._dropouts is None:   # found once: the key is computed on every forward
+            self._dropouts = self.findModules("nn.Dropout")
+        key = engine_key(input, self._dropouts)
         if self._engine is None or self._engine.key != key:
             # plans are kept per input shape (most recent MAX_ENGINES): the reference's loop alternates between the training
             # batch and the partial last batch of the test pass (pipelines/standard/test.lua:40-44) every epoch
@@ -443,9 +447,11 @@ class Dropout(Module):
         self.p = p
 
     def trace(self, x, b):
+        """training: y = x * mask / (1 - p), a fresh mask per forward (the lowered plan's DropOp); evaluate(): y = x"""
+        if not 0 <= self.p < 1:
+            raise ValueError(f"nn.Dropout: p = {self.p} is outside [0, 1)")
         if self.p > 0 and self.train:
-            raise NotImplementedError("nn.Dropout in training mode is outside the hot-path scope "
-                                      "(-isDropout defaults to false, models/cifar/rnmg.lua:455)")
+            return b.dropout(x, self.p)
         return x
 
 

@@ -12,7 +12,7 @@ import os
 import torch
 
 from . import ffi
-from .ffi import mg_grid, mg_conv_desc, mg_grad_src, mg_bn_fused, ptr, MG_SEG_SAME, MG_SEG_POOL, MG_SEG_UP, MG_SRC_POOL3, MG_MAX_SRC
+from .ffi import mg_grid, mg_conv_desc, mg_grad_src, mg_bn_fused, mg_dropout, ptr, MG_SEG_SAME, MG_SEG_POOL, MG_SEG_UP, MG_SRC_POOL3, MG_MAX_SRC
 
 
 def cpad(c):
@@ -697,6 +697,70 @@ class CatOp(Op):
     def bwd(self, E):
         if self.comb is not None:
             self.comb.run()
+
+
+class DropStepOp(Op):
+    """device counter of the plan's dropout masks, advanced on the stream once per training forward before the first DropOp:
+    a captured step (graph.GraphedStep) draws new masks on every replay"""
+
+    def setup_fwd(self, E):
+        self.step = E.alloc((1,), torch.int64)
+
+    def io_fwd(self):
+        return [], _keys(self.step)
+
+    def io_bwd(self):
+        return [], []
+
+    def fwd(self, E):
+        E.ctx.call("mg_dropout_advance", ptr(self.step))
+
+
+class DropOp(Op):
+    """nn.Dropout(p) in training mode in front of a convolution (models/cifar/pnmg.lua:25-27): the dropped concatenation of
+    the conv's segments, materialised as one tensor that the conv reads as its only segment.  Every element of an up-sampled
+    pixel has its own mask element, so the dropout cannot ride on the conv's gather.  Backward: the gradient of the dropped
+    tensor times the same mask (regenerated, in place), routed to the parts like CatOp's"""
+
+    def __init__(self, segs, p, ordinal, step_op, out):
+        self.segs, self.p, self.ordinal, self.step_op, self.out = segs, p, ordinal, step_op, out
+        out.producer = self
+
+    def setup_fwd(self, E):
+        self.out.buf = E.alloc(self.out.shape())
+        self.go = self.out.grid()
+        n = len(self.segs)
+        self.sg = (mg_grid * n)(*[t.grid() for t, _ in self.segs])
+        self.sm = (C.c_int32 * n)(*[m for _, m in self.segs])
+        self.dp = mg_dropout(self.p, self.ordinal, E.dropout_rank, E.dropout_seed, self.step_op.step.data_ptr())
+
+    def io_fwd(self):
+        return _keys(self.step_op.step, *[t.buf for t, _ in self.segs]), _keys(self.out.buf)
+
+    def io_bwd(self):
+        if self.comb is None:
+            return [], []
+        return _merge(self.comb.io(), (_keys(self.step_op.step, self.comb.buf), _keys(self.comb.buf)))
+
+    def fwd(self, E):
+        E.ctx.call("mg_dropout_forward", C.byref(self.dp), len(self.segs), self.sg, self.sm, C.byref(self.go))
+
+    def setup_bwd(self, E):
+        t = self.out
+        self.comb = None
+        if t.needs_grad:
+            self.comb = Combine(E, t)   # usually an alias of the consuming conv's dcat
+            self.dg = self.comb.grid()
+            off = 0
+            for p, m in self.segs:
+                if p.needs_grad:
+                    p.srcs.append(Src(self.comb.buf, t.H, t.W, t.C, t.Cp, off, m))
+                off += p.C
+
+    def bwd(self, E):
+        if self.comb is not None:
+            self.comb.run()
+            E.ctx.call("mg_dropout_backward", C.byref(self.dp), C.byref(self.dg))
 
 
 class GlobalAvgOp(Op):
