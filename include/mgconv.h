@@ -222,6 +222,8 @@ int mg_pool_forward(mg_ctx* ctx, const mg_grid* in, mg_grid* out, int32_t c_offs
 int mg_copy_channels(mg_ctx* ctx, const mg_grid* in, mg_grid* out, int32_t c_offset);
 /* cudnn.SpatialAveragePooling(r,r,r,r) on NHWC (image pyramid, rnmg.lua:175-177) */
 int mg_avgpool_forward(mg_ctx* ctx, const mg_grid* in, int32_t r, mg_grid* out);
+/* its backward (floor mode, divisor r*r): din[n][y][x][c] = dout[n][y/r][x/r][c] / (r*r), 0 in the rows / columns no window covers */
+int mg_avgpool_backward(mg_ctx* ctx, const mg_grid* dout, int32_t r, mg_grid* din);
 /* im2col of the image-fed stem convolution cudnn.SpatialConvolution(3, C, 7,7, 2,2, 3,3) (rnmg.lua:180):
  * col[n][oy][ox][ci*k*k + ky*k + kx] = in[n][oy*stride-pad+ky][ox*stride-pad+kx][ci].  The channel order is Torch's
  * [Cout][Cin][kH][kW] weight layout flattened, so the stem becomes a 1x1 mg_conv over `col` that uses the module's
@@ -285,8 +287,22 @@ int mg_bn_backward(mg_ctx* ctx, const mg_grid* xraw, const mg_grid* d, mg_grid* 
                    int64_t count, const float* gamma, const float* save_mean, const float* save_invstd,
                    float* dgamma, float* dbeta, float gscale, float* coef_ws /* [3*Cp] scratch */,
                    float* conv_dbias);
+/* Backward of a BatchNorm in evaluation mode ("frozen": it normalised with its running statistics and did not update them --
+ * model:evaluate(), or bn:evaluate() inside a training model).  It is then a fixed per-channel affine, so (THNN
+ * BatchNormalization_backward with train == false)
+ *      G = A * d,  A = gamma * invstd_r,  invstd_r = 1 / sqrt(running_var + eps)  (fp64, as mg_bn_finalize derives it),
+ * and no second pass over d is needed: mg_grad_combine_bn_frozen is mg_grad_combine (same x, relu_mask, bn_x, sources) that writes
+ * G = A * d to g, writes d itself only when d != NULL (a residual shortcut reads it), and accumulates (sum d, sum d*bn_x) into
+ * bn_sums[2*C] (required, caller zeroes).  gamma nullable (1).  mg_bn_backward_frozen turns the sums into the parameter gradients:
+ *      dgamma += gscale * invstd_r * (sum d*y - running_mean * sum d),  dbeta += gscale * sum d,
+ *      conv_dbias (nullable: gradBias of the convolution that produced y) += gscale * A * sum d. */
+int mg_grad_combine_bn_frozen(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int32_t n_src, const mg_grad_src* src,
+                              const float* gamma, const float* running_var, float eps, mg_grid* g, mg_grid* d, mg_sum* bn_sums);
+int mg_bn_backward_frozen(mg_ctx* ctx, const mg_sum* bn_sums, int32_t C, const float* gamma, const float* running_mean,
+                          const float* running_var, float eps, float* dgamma, float* dbeta, float gscale, float* conv_dbias);
 /* dcat = conv_transpose(g, w): gradient w.r.t. the concatenated input, segment s at channel
- * offset sum_{t<s} Cp_t */
+ * offset sum_{t<s} Cp_t.  Strided descriptors (the image-fed stem cudnn.SpatialConvolution(3, C, 7,7, 2,2, 3,3), rnmg.lua:180:
+ * one unresampled segment of at most 8 channels) run a CUDA-core kernel from the fp32 weights w in both dtypes; wpack_t is unused. */
 int mg_conv_backward_data(mg_ctx* ctx, const mg_conv_desc* d, const float* w, const void* wpack_t,
                           const mg_grid* g, mg_grid* dcat);
 /* dw += gscale * g^T * gather(x) ; dbias += gscale * sum(g)   (accGradParameters) */
@@ -325,7 +341,10 @@ size_t mg_plan_workspace_bytes(const mg_stage_plan* plan);
 int mg_plan_destroy(mg_stage_plan* plan);
 /* updateOutput: x[i] -> y[i] (NCHW fp32, [batch][C][H[i]][W[i]]); training != 0: batch statistics + running-statistics update */
 int mg_stage_forward(mg_stage_plan* plan, void* workspace, const float* const* x, const mg_stage_params* params, float* const* y, int training);
-/* updateGradInput + accGradParameters(scale): dy[i] -> dx[i] (dx or single entries may be NULL: no input gradient wanted) */
+/* updateGradInput + accGradParameters(scale): dy[i] -> dx[i] (dx or single entries may be NULL: no input gradient wanted).
+ * The BatchNorm backward follows the mode of the plan's last mg_stage_forward: after training = 0 every BatchNorm of the stage is
+ * differentiated in evaluation mode (running statistics, mg_grad_combine_bn_frozen / mg_bn_backward_frozen); after training != 0
+ * in training mode (batch statistics, mg_bn_backward).  Calling it before any mg_stage_forward is an error. */
 int mg_stage_backward(mg_stage_plan* plan, void* workspace, const float* const* dy, const mg_stage_params* params, float* const* dx, float scale);
 
 /* ---- head / criterion / optimiser ("next" rows of the scope table) ------------------- */

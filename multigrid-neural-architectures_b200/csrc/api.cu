@@ -10,6 +10,7 @@
 // simt_conv.cu
 int simt_conv_forward(mg_ctx*, const mg_conv_desc*, const float*, const float*, mg_grid*, mg_sum*);
 int simt_conv_backward_data(mg_ctx*, const mg_conv_desc*, const float*, const mg_grid*, mg_grid*);
+int simt_strided_dgrad(mg_ctx*, const mg_conv_desc*, const float*, const mg_grid*, mg_grid*);
 int simt_conv_backward_weight(mg_ctx*, const mg_conv_desc*, const mg_grid*, float*, float*, float);
 // umma_conv.cu
 bool umma_conv_supported(const mg_ctx*, const mg_conv_desc*, int kind);
@@ -237,6 +238,10 @@ int mg_conv_backward_data(mg_ctx* ctx, const mg_conv_desc* d, const float* w, co
   MG_REQUIRE(ctx, g->C == d->Cout, MG_ERR_SHAPE, "conv_backward_data: g.C %d != Cout %d", g->C, d->Cout);
   MG_REQUIRE(ctx, dcat->H == d->H && dcat->W == d->W && dcat->N == g->N, MG_ERR_SHAPE, "conv_backward_data: dcat shape");
   ProfSpan span(ctx);
+  if (d->stride != 1) {   // the image-fed strided stem: a CUDA-core kernel in every dtype and impl (simt_conv.cu: stem_dgrad_kernel)
+    MG_REQUIRE(ctx, w != nullptr, MG_ERR_INVALID_ARG, "conv_backward_data: null weights");
+    return simt_strided_dgrad(ctx, d, w, g, dcat);
+  }
   if (use_umma(ctx, d, wpack_t, 1)) return umma_conv_backward_data(ctx, d, wpack_t, g, dcat);
   MG_REQUIRE(ctx, ctx->impl != MG_IMPL_TCGEN05, MG_ERR_UNSUPPORTED, "conv_backward_data: shape not supported by the tcgen05 path");
   MG_REQUIRE(ctx, w != nullptr, MG_ERR_INVALID_ARG, "conv_backward_data: null weights");

@@ -267,6 +267,11 @@ __host__ __device__ __forceinline__ double mg_sum_get(const mg_sum& s) {
   return (double)s.hi * (1.0 / 1024.0) + (double)s.lo * (1.0 / 18014398509481984.0);   // 2^-54
 }
 
+// BatchNorm in evaluation mode ("frozen": running statistics, no update): invstd_r = 1 / sqrt(running_var + eps) in fp64, the
+// expression of mg_bn_finalize.  FrozenBn carries what mg_grad_combine_bn_frozen hands to the combine kernels.
+__device__ __forceinline__ double frozen_bn_invstd(float rvar, float eps) { return 1.0 / sqrt((double)rvar + (double)eps); }
+struct FrozenBn { const float* gamma; const float* running_var; float eps; const mg_grid* g; };
+
 // ---- programmatic dependent launch (PDL) ---------------------------------------------------------
 // A kernel launched with mg_launch_pdl may become resident while its predecessor in the stream is still
 // draining; it must execute pdl_wait() before touching anything the predecessor wrote.  pdl_launch() (first

@@ -11,7 +11,8 @@ int upconv_tc_forward(mg_ctx*, const mg_grid* x, const float* w, const float* bi
 int upconv_tc_backward(mg_ctx*, const mg_grid* x, const float* w, const mg_grid* g, mg_grid* dx, float* dw, float* dbias, float gscale);
 bool bf16_apply(mg_ctx*, const mg_grid* z, const mg_grid* s, int relu, mg_grid* out, mg_grid* pooled, const mg_bn_fused* bn);
 bool bf16_bn_stats(mg_ctx*, const mg_grid* y, mg_sum* sums);
-bool bf16_combine(mg_ctx*, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int n_src, const mg_grad_src* src, mg_grid* d, mg_sum* sums);
+bool bf16_combine(mg_ctx*, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int n_src, const mg_grad_src* src, mg_grid* d, mg_sum* sums,
+                  const FrozenBn* fz);
 bool bf16_bn_bwd_apply(mg_ctx*, const mg_grid* xraw, const mg_grid* d, mg_grid* out, const mg_sum* sums, int64_t count, const float* gamma,
                        const float* mean, const float* invstd, float* dgamma, float* dbeta, float* conv_dbias, float gscale);
 int simt_dbias(mg_ctx* ctx, const mg_grid* g, int Cout, float* dbias, float gscale);
@@ -195,6 +196,20 @@ __global__ void avgpool_kernel(GridV<T> in, int r, T* __restrict__ out, int Ho, 
   mg_st(out + i, s);
 }
 
+// backward of avgpool_kernel (floor mode, divisor r*r): every input pixel of a window receives dout / (r*r); rows and columns
+// beyond Ho*r / Wo*r belong to no window and receive 0
+template <typename T>
+__global__ void avgpool_bwd_kernel(GridV<T> dout, int r, T* __restrict__ din, int N, int H, int W, int C, int Cp) {
+  int64_t i = (int64_t)blockIdx.x * EB + threadIdx.x;
+  int64_t total = (int64_t)N * H * W * Cp;
+  if (i >= total) return;
+  int c = i % Cp; int64_t p = i / Cp;
+  int x = p % W; int64_t q = p / W; int y = q % H; int n = q / H;
+  float v = 0.f;
+  if (c < C && y / r < dout.H && x / r < dout.W) v = dout.raw(n, y / r, x / r, c) / (float)(r * r);
+  mg_st(din + i, v);
+}
+
 // SpatialMaxPooling(3,3,2,2,1,1): floor mode, windows clipped to the image
 template <typename T>
 __device__ __forceinline__ float pool3_window(const GridV<T>& in, int n, int oy, int ox, int c, int* arg) {
@@ -256,9 +271,11 @@ struct CombineP {
   int relu_mask;
   const T* bn_x; int bn_cp;
   int n_src; SrcV<T> src[MG_MAX_SRC];
-  T* d; int d_cp;
+  T* d; int d_cp;                // d may be null when g is set
   mg_sum* bn_sums;
   int pix_per_block;
+  // frozen BatchNorm (mg_grad_combine_bn_frozen): also g = gamma * invstd_r * d
+  T* g; int g_cp; const float* fz_gamma; const float* fz_rvar; float fz_eps;
 };
 
 // block = 32 channels x 8 pixel lanes
@@ -271,6 +288,8 @@ __global__ void __launch_bounds__(256) combine_kernel(CombineP<T> p) {
   const int64_t p1 = min(P, p0 + p.pix_per_block);
   const GridV<T>& X = p.x;
   float sd = 0.f, sdx = 0.f;
+  float A = 0.f;
+  if (p.g && c < X.C) A = (float)((p.fz_gamma ? (double)p.fz_gamma[c] : 1.0) * frozen_bn_invstd(p.fz_rvar[c], p.fz_eps));
   if (c < p.d_cp) {
     for (int64_t pix = p0 + lane; pix < p1; pix += 8) {
       float sum = 0.f;
@@ -301,7 +320,8 @@ __global__ void __launch_bounds__(256) combine_kernel(CombineP<T> p) {
         if (p.relu_mask) { float v = X.at(n, y, x, c); if (!(v > 0.f)) sum = 0.f; }
         if (p.bn_sums) { sd += sum; sdx += sum * mg_ld(p.bn_x + pix * p.bn_cp + c); }
       }
-      mg_st(p.d + pix * p.d_cp + c, sum);
+      if (p.d) mg_st(p.d + pix * p.d_cp + c, sum);
+      if (p.g) mg_st(p.g + pix * p.g_cp + c, A * sum);
     }
   }
   if (p.bn_sums) {
@@ -352,6 +372,23 @@ __global__ void bn_bwd_apply_kernel(const T* __restrict__ xraw, int x_cp, const 
   if (c < C)
     v = fmaf(coef[c], mg_ld(d + pix * d_cp + c), fmaf(coef[d_cp + c], mg_ld(xraw + pix * x_cp + c), coef[2 * d_cp + c]));
   mg_st(out + i, v);
+}
+
+// frozen BatchNorm: parameter gradients from the sums of mg_grad_combine_bn_frozen (fp64 from the fixed-point totals, no
+// floating-point atomics): dgamma += gscale * invstd_r * (sum d*y - mu_r * sum d), dbeta += gscale * sum d and the producing
+// convolution's gradBias += gscale * A * sum d (= the pixel sum of G = A * d)
+__global__ void bn_bwd_frozen_kernel(const mg_sum* sums, int C, const float* gamma, const float* rmean, const float* rvar, float eps,
+                                     float* dgamma, float* dbeta, float gscale, float* conv_dbias) {
+  pdl_launch();
+  pdl_wait();
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  const double sd = mg_sum_get(sums[c]), sdy = mg_sum_get(sums[C + c]);
+  const double is = frozen_bn_invstd(rvar[c], eps);
+  if (dgamma) dgamma[c] += gscale * (float)(is * (sdy - (double)rmean[c] * sd));
+  if (dbeta) dbeta[c] += gscale * (float)sd;
+  const float A = (float)((gamma ? (double)gamma[c] : 1.0) * is);
+  if (conv_dbias) conv_dbias[c] += gscale * (float)((double)A * sd);
 }
 
 // ---------------------------------------------------------------- input path: crop / flip / normalise ----------
@@ -692,6 +729,17 @@ int mg_avgpool_forward(mg_ctx* ctx, const mg_grid* in, int32_t r, mg_grid* out) 
   return MG_OK;
 }
 
+int mg_avgpool_backward(mg_ctx* ctx, const mg_grid* dout, int32_t r, mg_grid* din) {
+  if (!ctx || !dout || !din || !dout->data || !din->data || r < 1) return MG_ERR_INVALID_ARG;
+  MG_REQUIRE(ctx, dout->H == din->H / r && dout->W == din->W / r && dout->N == din->N && dout->C == din->C, MG_ERR_SHAPE,
+             "avgpool_backward: dout %dx%d for din %dx%d, r %d", dout->H, dout->W, din->H, din->W, r);
+  int64_t total = (int64_t)din->N * din->H * din->W * din->Cp;
+  MG_DISPATCH(ctx, avgpool_bwd_kernel<T><<<GRID1(total), EB, 0, ctx->stream>>>(make_view<T>(*dout), r, (T*)din->data, din->N, din->H, din->W,
+                                                                              din->C, din->Cp););
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
 int mg_pool3s2_forward(mg_ctx* ctx, const mg_grid* in, mg_grid* out, uint8_t* argmax_code) {
   if (!ctx || !in || !out) return MG_ERR_INVALID_ARG;
   int Ho = (in->H + 2 - 3) / 2 + 1, Wo = (in->W + 2 - 3) / 2 + 1;
@@ -721,20 +769,23 @@ int mg_global_avgpool_backward(mg_ctx* ctx, const mg_grid* dout, mg_grid* din) {
   return MG_OK;
 }
 
-int mg_grad_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int32_t n_src,
-                    const mg_grad_src* src, mg_grid* d, mg_sum* bn_sums) {
-  if (!ctx || !x || !d || n_src < 0 || n_src > MG_MAX_SRC || (n_src && !src)) return MG_ERR_INVALID_ARG;
+}  // extern "C"
+
+// mg_grad_combine, and with fz the frozen-BatchNorm form (mg_grad_combine_bn_frozen): `o` is the tensor written in full (d, or G)
+static int grad_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int32_t n_src, const mg_grad_src* src,
+                        mg_grid* d, mg_sum* bn_sums, const FrozenBn* fz) {
+  const mg_grid* o = fz ? fz->g : d;
   if (relu_mask == 2) {
     // the tensor itself was never stored (mg_bn_relu_pool3_forward): x is its 3x3 / stride-2 max-pooled form, the one source routes
     // through the arg-max codes, and the ReLU mask of an element is the sign of the pooled value it was the arg-max of
     MG_REQUIRE(ctx, n_src == 1 && src[0].mode == 3 && src[0].aux && bn_x, MG_ERR_INVALID_ARG, "combine: relu_mask 2 needs one arg-max-coded source and bn_x");
-    MG_REQUIRE(ctx, x->N == d->N && x->C == d->C && x->H == (d->H - 1) / 2 + 1 && x->W == (d->W - 1) / 2 + 1 && src[0].g.H == x->H && src[0].g.W == x->W
-               && bn_x->H == d->H && bn_x->W == d->W, MG_ERR_SHAPE, "combine: relu_mask 2 shapes");
-    MG_REQUIRE(ctx, ctx->dtype == MG_BF16 && bf16_combine(ctx, x, relu_mask, bn_x, n_src, src, d, bn_sums), MG_ERR_UNSUPPORTED, "combine: relu_mask 2 is a bf16 fast path");
+    MG_REQUIRE(ctx, x->N == o->N && x->C == o->C && x->H == (o->H - 1) / 2 + 1 && x->W == (o->W - 1) / 2 + 1 && src[0].g.H == x->H && src[0].g.W == x->W
+               && bn_x->H == o->H && bn_x->W == o->W, MG_ERR_SHAPE, "combine: relu_mask 2 shapes");
+    MG_REQUIRE(ctx, ctx->dtype == MG_BF16 && bf16_combine(ctx, x, relu_mask, bn_x, n_src, src, d, bn_sums, fz), MG_ERR_UNSUPPORTED, "combine: relu_mask 2 is a bf16 fast path");
     MG_CHECK_LAUNCH(ctx);
     return MG_OK;
   }
-  MG_REQUIRE(ctx, d->N == x->N && d->H == x->H && d->W == x->W && d->C == x->C, MG_ERR_SHAPE, "combine: d shape");
+  MG_REQUIRE(ctx, o->N == x->N && o->H == x->H && o->W == x->W && o->C == x->C, MG_ERR_SHAPE, "combine: d shape");
   for (int s = 0; s < n_src; ++s) {
     const mg_grid& g = src[s].g;
     int m = src[s].mode;
@@ -747,7 +798,7 @@ int mg_grad_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid*
     MG_REQUIRE(ctx, ok, MG_ERR_SHAPE, "combine: src %d (mode %d, %dx%dx%d off %d) does not match x %dx%dx%d", s, m, g.H,
                g.W, g.Cp, src[s].c_offset, x->H, x->W, x->C);
   }
-  if (ctx->dtype == MG_BF16 && bf16_combine(ctx, x, relu_mask, bn_x, n_src, src, d, bn_sums)) { MG_CHECK_LAUNCH(ctx); return MG_OK; }
+  if (ctx->dtype == MG_BF16 && bf16_combine(ctx, x, relu_mask, bn_x, n_src, src, d, bn_sums, fz)) { MG_CHECK_LAUNCH(ctx); return MG_OK; }
   int64_t P = (int64_t)x->N * x->H * x->W;
   MG_DISPATCH(ctx, {
     CombineP<T> p;
@@ -755,11 +806,39 @@ int mg_grad_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid*
     p.bn_x = (const T*)(bn_x ? bn_x->data : x->data); p.bn_cp = bn_x ? bn_x->Cp : x->Cp;
     p.n_src = n_src;
     for (int s = 0; s < n_src; ++s) { p.src[s].g = make_view<T>(src[s].g); p.src[s].c_off = src[s].c_offset; p.src[s].mode = src[s].mode; }
-    p.d = (T*)d->data; p.d_cp = d->Cp; p.bn_sums = bn_sums;
+    p.d = d ? (T*)d->data : nullptr; p.d_cp = o->Cp; p.bn_sums = bn_sums;
+    p.g = fz ? (T*)fz->g->data : nullptr; p.g_cp = o->Cp;
+    p.fz_gamma = fz ? fz->gamma : nullptr; p.fz_rvar = fz ? fz->running_var : nullptr; p.fz_eps = fz ? fz->eps : 0.f;
     p.pix_per_block = 64;
-    dim3 grid((unsigned)mg_cdiv(P, p.pix_per_block), (unsigned)mg_cdiv(d->Cp, 32));
+    dim3 grid((unsigned)mg_cdiv(P, p.pix_per_block), (unsigned)mg_cdiv(o->Cp, 32));
     combine_kernel<T><<<grid, 256, 0, ctx->stream>>>(p);
   });
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
+extern "C" {
+
+int mg_grad_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int32_t n_src,
+                    const mg_grad_src* src, mg_grid* d, mg_sum* bn_sums) {
+  if (!ctx || !x || !d || n_src < 0 || n_src > MG_MAX_SRC || (n_src && !src)) return MG_ERR_INVALID_ARG;
+  return grad_combine(ctx, x, relu_mask, bn_x, n_src, src, d, bn_sums, nullptr);
+}
+
+int mg_grad_combine_bn_frozen(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int32_t n_src, const mg_grad_src* src,
+                              const float* gamma, const float* running_var, float eps, mg_grid* g, mg_grid* d, mg_sum* bn_sums) {
+  if (!ctx || !x || !bn_x || !running_var || !g || !bn_sums || n_src < 0 || n_src > MG_MAX_SRC || (n_src && !src)) return MG_ERR_INVALID_ARG;
+  MG_REQUIRE(ctx, bn_x->N == g->N && bn_x->H == g->H && bn_x->W == g->W && bn_x->C == g->C, MG_ERR_SHAPE, "combine_bn_frozen: bn_x shape");
+  if (d) MG_REQUIRE(ctx, d->N == g->N && d->H == g->H && d->W == g->W && d->C == g->C && d->Cp == g->Cp, MG_ERR_SHAPE, "combine_bn_frozen: d shape");
+  const FrozenBn fz = {gamma, running_var, eps, g};
+  return grad_combine(ctx, x, relu_mask, bn_x, n_src, src, d, bn_sums, &fz);
+}
+
+int mg_bn_backward_frozen(mg_ctx* ctx, const mg_sum* bn_sums, int32_t C, const float* gamma, const float* running_mean, const float* running_var,
+                          float eps, float* dgamma, float* dbeta, float gscale, float* conv_dbias) {
+  if (!ctx || !bn_sums || !running_mean || !running_var || C < 1) return MG_ERR_INVALID_ARG;
+  mg_launch_pdl(bn_bwd_frozen_kernel, dim3((unsigned)mg_cdiv(C, 128)), dim3(128), 0, ctx->stream, bn_sums, (int)C, gamma, running_mean, running_var,
+                eps, dgamma, dbeta, gscale, conv_dbias);
   MG_CHECK_LAUNCH(ctx);
   return MG_OK;
 }

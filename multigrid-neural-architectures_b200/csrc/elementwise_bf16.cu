@@ -290,6 +290,10 @@ struct CombP {
   mg_sum* sums;
   int N, H, W, C, Hb, Wb;        // Hb = ceil(H/2): 2x2 blocks
   FastDiv fd_wb, fd_hb;          // combine_fast_kernel: index decode
+  // frozen BatchNorm (combine_fast_kernel<.., true>): G = A * d with A = gamma * invstd_r derived per CTA; d is stored only when
+  // p.d is set (a residual shortcut reads it)
+  const float* fz_gamma; const float* fz_rvar; float fz_eps;
+  bf16* g; int g_cp;
 };
 
 // NS >= 0: the number of sources and their modes (2 bits each in MODES) are compile-time constants, so the source loop
@@ -431,8 +435,15 @@ __global__ void __launch_bounds__(256, NS < 0 ? 3 : 2) combine_bf16_kernel(const
 // chain of dependent ones (the older form above reuses one destination register for consecutive loads and interleaves the
 // BatchNorm-input loads with the stores: ~13 round trips per block).  Pixels outside the grid (odd H / W) re-read pixel 0 of
 // the block and are dropped at the store.  Same arithmetic and summation order as combine_bf16_kernel.
-template <int NS, int MODES>
-__global__ void __launch_bounds__(256, 2) combine_fast_kernel(const __grid_constant__ CombP p) {
+//
+// FROZEN: the tensor feeds a BatchNorm in evaluation mode, a fixed per-channel affine, so its backward is G = A * d with
+// A = gamma * invstd_r (frozen_bn_invstd, as mg_bn_finalize derives it from the running variance).  The same pass writes G
+// (and d only when p.d is set), still accumulating (sum d, sum d*y) for dgamma / dbeta (mg_bn_backward_frozen): no second pass
+// over d and y.
+// The frozen form keeps the batched loads of its 2x2 block AND the product with A live at once: at two CTAs per SM (128 registers)
+// the longer source lists spill, so it runs one CTA per SM with the whole register budget.
+template <int NS, int MODES, bool FROZEN>
+__global__ void __launch_bounds__(256, FROZEN ? 1 : 2) combine_fast_kernel(const __grid_constant__ CombP p) {
   pdl_launch();
   pdl_wait();
   extern __shared__ float sh[];
@@ -451,6 +462,12 @@ __global__ void __launch_bounds__(256, 2) combine_fast_kernel(const __grid_const
                             (((MODES >> 6) & 3) == 1 && NS > 3);
   const bool need_x = p.relu_mask == 1 || any_pool;   // relu_mask == 2: x is the POOLED tensor of the single mode-3 source (stem)
   const bool has_sums = p.sums != nullptr;
+  float* s_a = sh + 2 * 256 * 8;   // FROZEN: A per channel, after the block_channel_sums staging (read at the store: no registers held)
+  if (FROZEN) {
+    for (int c = threadIdx.x; c < p.g_cp; c += blockDim.x)
+      s_a[c] = c < p.C ? (float)((p.fz_gamma ? (double)p.fz_gamma[c] : 1.0) * frozen_bn_invstd(p.fz_rvar[c], p.fz_eps)) : 0.f;
+    __syncthreads();
+  }
 
   if (active)
     for (uint32_t blk = b_begin + lane; blk < b_end; blk += lanes) {
@@ -596,7 +613,13 @@ __global__ void __launch_bounds__(256, 2) combine_fast_kernel(const __grid_const
 #pragma unroll
             for (int e = 0; e < 8; ++e) { sd[e] += acc[k].v[e]; sdx[e] = fmaf(acc[k].v[e], yr.v[e], sdx[e]); }
           }
-          *reinterpret_cast<uint4*>(p.d + (size_t)pix[k] * p.d_cp + c0) = pack8(acc[k]);
+          if (!FROZEN || p.d) *reinterpret_cast<uint4*>(p.d + (size_t)pix[k] * p.d_cp + c0) = pack8(acc[k]);
+          if (FROZEN) {
+            V8 gk;
+#pragma unroll
+            for (int e = 0; e < 8; ++e) gk.v[e] = s_a[c0 + e] * acc[k].v[e];
+            *reinterpret_cast<uint4*>(p.g + (size_t)pix[k] * p.g_cp + c0) = pack8(gk);
+          }
         }
     }
   if (p.sums) block_channel_sums(sd, sdx, vc, V, p.C, active, p.sums, sh);
@@ -965,15 +988,17 @@ bool bf16_bn_stats(mg_ctx* ctx, const mg_grid* y, mg_sum* sums) {
 }
 
 bool bf16_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* bn_x, int n_src, const mg_grad_src* src, mg_grid* d,
-                  mg_sum* sums) {
-  if (x->Cp % 8 || d->Cp % 8 || d->Cp > 2048 || x->scale || x->Cp < d->Cp) return false;
+                  mg_sum* sums, const FrozenBn* fz) {
+  const mg_grid* o = fz ? fz->g : d;   // the tensor the pass writes in full (G when frozen; d may then be null)
+  if (x->Cp % 8 || o->Cp % 8 || o->Cp > 2048 || x->scale || x->Cp < o->Cp) return false;
+  if (fz && d && d->Cp != o->Cp) return false;
   if (relu_mask == 2 && !(n_src == 1 && src[0].mode == 3 && src[0].aux && bn_x)) return false;   // x = pooled tensor of the stem's mode-3 source
-  if (sums && bn_x && bn_x->Cp < d->Cp) return false;
+  if (sums && bn_x && bn_x->Cp < o->Cp) return false;
   CombP p;
   memset(&p, 0, sizeof(p));
   for (int s = 0; s < n_src; ++s) {
     const mg_grad_src& g = src[s];
-    if (g.c_offset % 8 || g.g.Cp % 8 || g.c_offset + d->Cp > g.g.Cp) return false;
+    if (g.c_offset % 8 || g.g.Cp % 8 || g.c_offset + o->Cp > g.g.Cp) return false;
     if (g.mode == 3 && !g.aux) return false;
     p.src[s].g = (const bf16*)g.g.data; p.src[s].aux = (const uint8_t*)g.aux;
     p.src[s].H = g.g.H; p.src[s].W = g.g.W; p.src[s].cp = g.g.Cp; p.src[s].c_off = g.c_offset; p.src[s].mode = g.mode;
@@ -982,9 +1007,11 @@ bool bf16_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* b
   p.x = (const bf16*)x->data; p.x_cp = x->Cp;
   const mg_grid* bx = bn_x ? bn_x : x;
   p.bnx = (const bf16*)bx->data; p.bn_cp = bx->Cp;
-  p.relu_mask = relu_mask; p.d = (bf16*)d->data; p.d_cp = d->Cp; p.sums = sums;
-  p.N = d->N; p.H = d->H; p.W = d->W; p.C = d->C; p.Hb = (d->H + 1) / 2; p.Wb = (d->W + 1) / 2;
-  const int V = d->Cp / 8;
+  p.relu_mask = relu_mask; p.d = d ? (bf16*)d->data : nullptr; p.d_cp = o->Cp; p.sums = sums;
+  p.g = fz ? (bf16*)fz->g->data : nullptr; p.g_cp = o->Cp;
+  if (fz) { p.fz_gamma = fz->gamma; p.fz_rvar = fz->running_var; p.fz_eps = fz->eps; }
+  p.N = o->N; p.H = o->H; p.W = o->W; p.C = o->C; p.Hb = (o->H + 1) / 2; p.Wb = (o->W + 1) / 2;
+  const int V = o->Cp / 8;
   const int64_t items = (int64_t)p.N * p.Hb * p.Wb * V;
   static int spec = -1;
   if (spec < 0) { const char* e = getenv("MGCONV_COMBINE_SPEC"); spec = e ? atoi(e) : 1; }
@@ -997,11 +1024,16 @@ bool bf16_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* b
   for (int s = 0; s < n_src; ++s) code |= (src[s].mode & 3) << (2 * s);
   const size_t smem = sums ? 2 * 256 * 8 * sizeof(float) : 0;   // block_channel_sums staging
   // the source-mode lists of the multigrid builders (same / pool / up gathers of ResampleConcat + shortcut); anything else
-  // takes the generic kernel
+  // takes the generic kernel.  Frozen BatchNorm: the specialised batched-load kernels only (false otherwise: the caller then runs
+  // the generic kernel of elementwise.cu)
+  if (fz && !(spec && fast)) return false;
 #define MG_COMBINE_CASE(NSRC, M0, M1, M2, M3)                                                                      \
   if (spec && n_src == NSRC && code == ((M0) | (M1) << 2 | (M2) << 4 | (M3) << 6)) {                                  \
-    if (fast)                                                                                                        \
-      mg_launch_pdl(combine_fast_kernel<NSRC, ((M0) | (M1) << 2 | (M2) << 4 | (M3) << 6)>, dim3(reduce_grid(ctx, items, 2)), \
+    if (fz)                                                                                                          \
+      mg_launch_pdl(combine_fast_kernel<NSRC, ((M0) | (M1) << 2 | (M2) << 4 | (M3) << 6), true>, dim3(reduce_grid(ctx, items, 1)), \
+                    dim3(256), 2 * 256 * 8 * sizeof(float) + o->Cp * sizeof(float), ctx->stream, p);                \
+    else if (fast)                                                                                                   \
+      mg_launch_pdl(combine_fast_kernel<NSRC, ((M0) | (M1) << 2 | (M2) << 4 | (M3) << 6), false>, dim3(reduce_grid(ctx, items, 2)), \
                     dim3(256), smem, ctx->stream, p);                                                                \
     else                                                                                                             \
       mg_launch_pdl(combine_bf16_kernel<NSRC, ((M0) | (M1) << 2 | (M2) << 4 | (M3) << 6)>, dim3(reduce_grid(ctx, items, 2)), \
@@ -1020,6 +1052,7 @@ bool bf16_combine(mg_ctx* ctx, const mg_grid* x, int relu_mask, const mg_grid* b
   MG_COMBINE_CASE(3, 0, 2, 1, 0)
   MG_COMBINE_CASE(4, 0, 0, 2, 1)
 #undef MG_COMBINE_CASE
+  if (fz) return false;
   const unsigned grid = reduce_grid(ctx, items, 3);   // 80 registers: three CTAs per SM are resident
   mg_launch_pdl(combine_bf16_kernel<-1, 0>, dim3(grid), dim3(256), smem, ctx->stream, p);
   return true;

@@ -293,7 +293,7 @@ static int simt_dgrad_t(mg_ctx* ctx, const mg_conv_desc* d, const float* w, cons
   DgradProb<T> p;
   int rc = make_conv_view<T>(ctx, *d, &p.cv);
   if (rc) return rc;
-  MG_REQUIRE(ctx, d->stride == 1, MG_ERR_UNSUPPORTED, "dgrad: stride must be 1");
+  MG_REQUIRE(ctx, d->stride == 1, MG_ERR_UNSUPPORTED, "dgrad: stride %d goes through simt_strided_dgrad", d->stride);
   p.w = w; p.g = (const T*)g->data; p.g_cp = g->Cp; p.dcat = (T*)dcat->data;
   p.M = (int64_t)p.cv.N * p.cv.H * p.cv.W;
   MG_REQUIRE(ctx, dcat->Cp == p.cv.CcatP, MG_ERR_SHAPE, "dgrad: dcat.Cp %d != %d", dcat->Cp, p.cv.CcatP);
@@ -305,6 +305,77 @@ static int simt_dgrad_t(mg_ctx* ctx, const mg_conv_desc* d, const float* w, cons
 
 int simt_conv_backward_data(mg_ctx* ctx, const mg_conv_desc* d, const float* w, const mg_grid* g, mg_grid* dcat) {
   MG_DISPATCH(ctx, return simt_dgrad_t<T>(ctx, d, w, g, dcat););
+}
+
+// Data gradient of the image-fed strided stem, cudnn.SpatialConvolution(3, C, 7,7, 2,2, 3,3) (models/ilsvrc/rnmg.lua:180):
+//   dx[n][iy][ix][ci] = sum over (ky, kx) with iy = oy*stride - pad + ky, ix = ox*stride - pad + kx, and over co, of
+//                       g[n][oy][ox][co] * w[co][ci][ky][kx].
+// A CUDA-core kernel, not a tcgen05 one: the output has 3 channels (one 8-channel vector), far below the N >= 16 of an MMA, while
+// the reduction (49 taps x Cout) is long.  The whole fp32 weight tensor sits in shared memory as [ky][kx][co][ci]; one thread owns
+// one input pixel, visits only the taps of its parity class ((iy + pad - ky) divisible by the stride: 16 of 49 for 7x7 / 2) and
+// accumulates its <= 8 channels in registers in a fixed order, so the result is deterministic.
+template <typename T>
+__global__ void __launch_bounds__(128) stem_dgrad_kernel(const T* __restrict__ g, int g_cp, int Ho, int Wo, int Cout, const float* __restrict__ w,
+                                                         int Cin, int k, int stride, int pad, T* __restrict__ dx, int dx_cp, int N, int H, int W) {
+  extern __shared__ float s_w[];
+  const int taps = k * k;
+  for (int i = threadIdx.x; i < taps * Cout * Cin; i += blockDim.x) {
+    const int ci = i % Cin, r = i / Cin, co = r % Cout, t = r / Cout;
+    s_w[i] = w[((size_t)co * Cin + ci) * taps + t];
+  }
+  __syncthreads();
+  const int64_t P = (int64_t)N * H * W;
+  for (int64_t pix = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; pix < P; pix += (int64_t)gridDim.x * blockDim.x) {
+    const int ix = (int)(pix % W);
+    const int64_t q = pix / W;
+    const int iy = (int)(q % H), n = (int)(q / H);
+    float acc[8];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) acc[c] = 0.f;
+    for (int ky = (iy + pad) % stride; ky < k; ky += stride) {
+      const int oy = (iy + pad - ky) / stride;   // exact: iy + pad - ky is a multiple of the stride
+      if (iy + pad - ky < 0 || oy >= Ho) continue;
+      for (int kx = (ix + pad) % stride; kx < k; kx += stride) {
+        const int ox = (ix + pad - kx) / stride;
+        if (ix + pad - kx < 0 || ox >= Wo) continue;
+        const T* gp = g + (((size_t)n * Ho + oy) * Wo + ox) * g_cp;
+        const float* wp = s_w + (size_t)(ky * k + kx) * Cout * Cin;
+        for (int co = 0; co < Cout; ++co) {
+          const float gv = mg_ld(gp + co);
+#pragma unroll
+          for (int ci = 0; ci < 8; ++ci)
+            if (ci < Cin) acc[ci] = fmaf(gv, wp[co * Cin + ci], acc[ci]);
+        }
+      }
+    }
+    T* o = dx + pix * dx_cp;
+#pragma unroll
+    for (int c = 0; c < 8; ++c)
+      if (c < dx_cp) mg_st(o + c, c < Cin ? acc[c] : 0.f);
+  }
+}
+
+template <typename T>
+static int stem_dgrad_t(mg_ctx* ctx, const mg_conv_desc* d, const float* w, const mg_grid* g, mg_grid* dcat) {
+  const mg_grid& x = d->seg[0];
+  MG_REQUIRE(ctx, d->n_seg == 1 && d->seg_mode[0] == MG_SEG_SAME && !x.scale && x.C <= 8 && x.Cp == 8 && dcat->Cp == 8, MG_ERR_UNSUPPORTED,
+             "dgrad: a strided convolution needs one unresampled input of at most 8 channels (the image-fed stem)");
+  const int Ho = (d->H + 2 * d->pad - d->ksize) / d->stride + 1, Wo = (d->W + 2 * d->pad - d->ksize) / d->stride + 1;
+  MG_REQUIRE(ctx, g->H == Ho && g->W == Wo && g->N == x.N && dcat->N == x.N, MG_ERR_SHAPE, "dgrad: g is %dx%d, expected %dx%d", g->H, g->W, Ho, Wo);
+  const size_t smem = (size_t)d->ksize * d->ksize * d->Cout * x.C * sizeof(float);
+  MG_REQUIRE(ctx, smem <= 200 * 1024, MG_ERR_UNSUPPORTED, "dgrad: strided weights of %zu bytes exceed shared memory", smem);
+  if (smem > 48 * 1024)
+    MG_CUDA(ctx, cudaFuncSetAttribute(stem_dgrad_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int64_t P = (int64_t)x.N * d->H * d->W;
+  const unsigned grid = (unsigned)std::min<int64_t>(mg_cdiv(P, (int64_t)128), (int64_t)ctx->num_sms * 8);
+  stem_dgrad_kernel<T><<<grid, 128, smem, ctx->stream>>>((const T*)g->data, g->Cp, Ho, Wo, d->Cout, w, x.C, d->ksize, d->stride, d->pad,
+                                                         (T*)dcat->data, dcat->Cp, x.N, d->H, d->W);
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
+int simt_strided_dgrad(mg_ctx* ctx, const mg_conv_desc* d, const float* w, const mg_grid* g, mg_grid* dcat) {
+  MG_DISPATCH(ctx, return stem_dgrad_t<T>(ctx, d, w, g, dcat););
 }
 
 template <typename T>

@@ -15,6 +15,7 @@ struct mg_stage_plan {
   mg_ctx* ctx;
   mg_stage_desc d;
   int batch, n, layers, elt;
+  int last_training;   // training flag of the last mg_stage_forward (-1: none yet); mg_stage_backward differentiates that mode
   // byte offsets into the workspace
   size_t X[MG_STAGE_MAX_GRIDS], PX[MG_STAGE_MAX_GRIDS], DX[MG_STAGE_MAX_GRIDS], DY[MG_STAGE_MAX_GRIDS];
   size_t y[2][MG_STAGE_MAX_GRIDS], a[2][MG_STAGE_MAX_GRIDS], Pa[2][MG_STAGE_MAX_GRIDS];
@@ -85,6 +86,7 @@ int mg_plan_create(mg_ctx* ctx, const mg_stage_desc* d, int32_t batch, mg_stage_
   memset(p, 0, sizeof(*p));
   p->ctx = ctx; p->d = *d; p->batch = batch; p->n = d->n_scales; p->layers = d->residual ? 2 : 1;
   p->elt = (int)mg_elt_size(ctx->dtype);
+  p->last_training = -1;
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += al(bytes); return o; };
   const int n = p->n, L = p->layers;
@@ -149,6 +151,7 @@ int mg_stage_forward(mg_stage_plan* p, void* workspace, const float* const* x, c
   char* ws = (char*)workspace;
   MG_REQUIRE(ctx, ((uintptr_t)workspace & 255) == 0, MG_ERR_INVALID_ARG, "stage_forward: workspace must be 256-byte aligned");
   MG_TRY(mg_memset_zero(ctx, ws + p->sums_begin, p->sums_bytes));
+  p->last_training = training ? 1 : 0;
   // inputs: NCHW fp32 -> grids, plus the pooled companion every coarser neighbour gathers
   for (int i = 0; i < n; ++i) {
     MG_REQUIRE(ctx, x[i] != nullptr, MG_ERR_INVALID_ARG, "stage_forward: x[%d] is null", i);
@@ -171,7 +174,8 @@ int mg_stage_forward(mg_stage_plan* p, void* workspace, const float* const* x, c
       if (wp) MG_TRY(mg_conv_pack_weights(ctx, &cd, prm->conv_w[k], wp, 0));
       mg_grid Y = grid_of(ws, p->y[l][i], B, d.H[i], d.W[i], d.C_out[i]);
       mg_sum* sums = (mg_sum*)(ws + p->fsums[l][i]);
-      MG_TRY(mg_conv_forward(ctx, &cd, prm->conv_w[k], wp, prm->conv_b[k], &Y, sums));
+      // evaluation mode normalises with the running statistics: the epilogue reduces no batch statistics
+      MG_TRY(mg_conv_forward(ctx, &cd, prm->conv_w[k], wp, prm->conv_b[k], &Y, training ? sums : nullptr));
       // SpatialBatchNormalization -> [CAddTable with the (padded) shortcut] -> [ReLU] -> [pooled companion], one pass
       mg_grid Z = grid_of(ws, p->y[l][i], B, d.H[i], d.W[i], d.C_out[i], (const float*)(ws + p->scale[l][i]), (const float*)(ws + p->shift[l][i]));
       mg_bn_fused f;
@@ -202,6 +206,8 @@ int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy,
   const mg_stage_desc& d = p->d;
   const int n = p->n, L = p->layers, B = p->batch;
   char* ws = (char*)workspace;
+  MG_REQUIRE(ctx, p->last_training >= 0, MG_ERR_INVALID_ARG, "stage_backward: no mg_stage_forward on this plan yet");
+  const bool frozen = p->last_training == 0;
   for (int i = 0; i < n; ++i) {
     MG_REQUIRE(ctx, dy[i] != nullptr, MG_ERR_INVALID_ARG, "stage_backward: dy[%d] is null", i);
     mg_grid DY = grid_of(ws, p->DY[i], B, d.H[i], d.W[i], d.C_out[i]);
@@ -241,9 +247,15 @@ int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy,
       mg_sum* bs = (mg_sum*)(ws + p->bsums[l][i]);
       MG_TRY(mg_memset_zero(ctx, bs, 2 * (size_t)d.C_out[i] * sizeof(mg_sum)));
       const int relu = last ? (d.no_final_relu ? 0 : 1) : 1;
-      MG_TRY(mg_grad_combine(ctx, &A, relu, &Yraw, ns, src, &Dg, bs));
-      MG_TRY(mg_bn_backward(ctx, &Yraw, &Dg, &Gg, bs, (int64_t)B * d.H[i] * d.W[i], prm->bn_g[k], (const float*)(ws + p->mean[l][i]),
-                            (const float*)(ws + p->invstd[l][i]), prm->bn_gg[k], prm->bn_gb[k], scale, (float*)(ws + p->coef[l][i]), prm->conv_gb[k]));
+      if (frozen) {   // evaluation-mode BatchNorm: G = gamma * invstd_r * D in the combine pass; D itself only for the shortcut
+        MG_TRY(mg_grad_combine_bn_frozen(ctx, &A, relu, &Yraw, ns, src, prm->bn_g[k], prm->bn_rv[k], d.eps, &Gg, (last && d.residual) ? &Dg : nullptr, bs));
+        MG_TRY(mg_bn_backward_frozen(ctx, bs, d.C_out[i], prm->bn_g[k], prm->bn_rm[k], prm->bn_rv[k], d.eps, prm->bn_gg[k], prm->bn_gb[k], scale,
+                                     prm->conv_gb[k]));
+      } else {
+        MG_TRY(mg_grad_combine(ctx, &A, relu, &Yraw, ns, src, &Dg, bs));
+        MG_TRY(mg_bn_backward(ctx, &Yraw, &Dg, &Gg, bs, (int64_t)B * d.H[i] * d.W[i], prm->bn_g[k], (const float*)(ws + p->mean[l][i]),
+                              (const float*)(ws + p->invstd[l][i]), prm->bn_gg[k], prm->bn_gb[k], scale, (float*)(ws + p->coef[l][i]), prm->conv_gb[k]));
+      }
       mg_conv_desc cd;
       make_desc(p, ws, l, i, &cd);
       MG_TRY(mg_conv_backward_weight(ctx, &cd, &Gg, prm->conv_gw[k], nullptr, scale));

@@ -35,15 +35,19 @@ def _flatten(x):
     return [x]
 
 
-def engine_key(input, dropouts=()):
+def engine_key(input, dropouts=(), batchnorms=(), training=True):
     """plans are kept per input shape and device; a model with an active nn.Dropout (`dropouts`: its nn.Dropout modules) also
-    gets one plan per mode (training plans hold the dropout ops, evaluation plans are those of the same model without them)"""
+    gets one plan per mode (training plans hold the dropout ops, evaluation plans are those of the same model without them).
+    A training model whose BatchNorm modules (`batchnorms`) do not all train -- some frozen by bn:evaluate() -- gets one plan per
+    pattern of frozen layers; models in one mode keep the key of their input alone."""
     ts = _flatten(input)
     key = (tuple(input.shape) if isinstance(input, torch.Tensor) else tuple(tuple(t.shape) for t in ts),
            ts[0].device.index)
     active = [m for m in dropouts if m.p > 0]
     if active:
         key += (any(m.train for m in active),)
+    if training and not all(m.train for m in batchnorms):
+        key += (("frozen_bn",) + tuple(i for i, m in enumerate(batchnorms) if not m.train),)
     return key
 
 
@@ -56,7 +60,7 @@ class Engine:
                                   "call model:cuda() and move the inputs with put2GPU first")
         self.model = model
         self.device = inputs[0].device
-        self.key = engine_key(input, model.findModules("nn.Dropout"))
+        self.key = engine_key(input, model.findModules("nn.Dropout"), model.findModules("nn.SpatialBatchNormalization"), model.train)
         precision = getattr(model, "precision", os.environ.get("MGCONV_PRECISION", "bf16"))
         self.dtype, self.elt = _PRECISION[precision]
         self.ctx = ffi.Context(self.device.index, torch.cuda.current_stream(self.device).cuda_stream, self.dtype)
@@ -97,6 +101,7 @@ class Engine:
         self._dropout_rank = 0
         self.input_ops = [o for o in b.ops if isinstance(o, ops.InputOp)]
         self.conv_ops = [o for o in b.ops if isinstance(o, ops.ConvOp)]
+        self.bn_ops = [o for o in b.ops if isinstance(o, ops.ApplyOp) and o.bn is not None]
         ops.fuse_stem_pool3(b.ops, self)
         for o in b.ops:
             o.setup_fwd(self)
@@ -192,6 +197,10 @@ class Engine:
     def forward(self, input, training=True):
         self._bind_stream()
         self.training = training
+        # a BatchNorm trains only when the model trains and its own module does (Torch7: bn:evaluate() inside model:training());
+        # a frozen one normalises with its running statistics, leaves them alone, and is differentiated as that fixed affine
+        for o in self.bn_ops:
+            o.frozen = not (training and o.bn.train)
         for op, t in zip(self.input_ops, _flatten(input)):
             op.src = t.contiguous().float()
         self.pack_weights()
@@ -241,13 +250,13 @@ class Engine:
                 j += 1
             run = oplist[i:j]
             if fwd:
-                synced = self._allreduce_sums([a.conv.sums for a in run if a.bn is not None])
+                synced = self._allreduce_sums([a.conv.sums for a in run if a.bn is not None and not a.frozen])
                 for a in run:
                     a.fwd(self, synced=synced)
             else:
                 for a in run:
                     a.bwd_combine(self)
-                synced = self._allreduce_sums([a.dsums for a in run if a.bn is not None])
+                synced = self._allreduce_sums([a.dsums for a in run if a.bn is not None and not a.frozen])
                 for a in run:
                     a.bwd_bn(self, synced=synced)
             i = j

@@ -110,6 +110,7 @@ SIGNATURES = {
     "mg_pool_forward": (_I, [_P, _G, _G, C.c_int32, _P]),
     "mg_copy_channels": (_I, [_P, _G, _G, C.c_int32]),
     "mg_avgpool_forward": (_I, [_P, _G, C.c_int32, _G]),
+    "mg_avgpool_backward": (_I, [_P, _G, C.c_int32, _G]),
     "mg_im2col": (_I, [_P, _G, C.c_int32, C.c_int32, C.c_int32, _G]),
     "mg_pool3s2_forward": (_I, [_P, _G, _G, _P]),
     "mg_bn_relu_pool3_forward": (_I, [_P, _G, C.POINTER(mg_bn_fused), _G, _P]),
@@ -122,6 +123,8 @@ SIGNATURES = {
     "mg_dropout_advance": (_I, [_P, _P]),
     "mg_grad_combine": (_I, [_P, _G, _I, _G, C.c_int32, C.POINTER(mg_grad_src), _G, _P]),
     "mg_bn_backward": (_I, [_P, _G, _G, _G, _P, _I64, _P, _P, _P, _P, _P, _F, _P, _P]),
+    "mg_grad_combine_bn_frozen": (_I, [_P, _G, _I, _G, C.c_int32, C.POINTER(mg_grad_src), _P, _P, _F, _G, _G, _P]),
+    "mg_bn_backward_frozen": (_I, [_P, _P, C.c_int32, _P, _P, _P, _F, _P, _P, _F, _P]),
     "mg_conv_backward_data": (_I, [_P, _D, _P, _P, _G, _G]),
     "mg_conv_backward_weight": (_I, [_P, _D, _G, _P, _P, _F]),
     "mg_nll_forward_backward": (_I, [_P, _G, _P, _P, _P, _G, _F]),

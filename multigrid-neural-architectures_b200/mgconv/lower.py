@@ -244,10 +244,8 @@ class Builder:
 
     def avgpool(self, v, k, d):
         t = self.as_tensor(v).spec
-        if k == d:  # image pyramid (ilsvrc/rnmg.lua:175-177)
-            if t.needs_grad:
-                raise NotImplementedError("SpatialAveragePooling(r,r,r,r) is only lowered on the input image")
-            out = self.new_tensor(t.C, t.H // k, t.W // k, f"{t.name}.avg{k}", needs_grad=False)
+        if k == d:  # image pyramid (ilsvrc/rnmg.lua:175-177): carries a gradient when the image does (needInputGrad)
+            out = self.new_tensor(t.C, t.H // k, t.W // k, f"{t.name}.avg{k}", needs_grad=t.needs_grad)
             self.emit(O.AvgPoolOp(t, k, out))
             return TVal(out)
         if d == 1 and k == t.H and k == t.W:  # classifier head Avg(7,7,1,1) on the 7x7 grid (rnmg.lua:282)

@@ -33,6 +33,7 @@ class Module:
         self.gradInput = None
         self._engine = None
         self._dropouts = None
+        self._batchnorms = None
 
     # ---- graph walking ----------------------------------------------------------------
     def children(self):
@@ -121,6 +122,7 @@ class Module:
             m._engine = None
             m._engines = None
             m._dropouts = None
+            m._batchnorms = None
             m.output = None
             m.gradInput = None
         return self
@@ -131,7 +133,8 @@ class Module:
         from .engine import engine_key
         if self._dropouts is None:   # found once: the key is computed on every forward
             self._dropouts = self.findModules("nn.Dropout")
-        key = engine_key(input, self._dropouts)
+            self._batchnorms = self.findModules("nn.SpatialBatchNormalization")
+        key = engine_key(input, self._dropouts, self._batchnorms, self.train)
         if self._engine is None or self._engine.key != key:
             # plans are kept per input shape (most recent MAX_ENGINES): the reference's loop alternates between the training
             # batch and the partial last batch of the test pass (pipelines/standard/test.lua:40-44) every epoch

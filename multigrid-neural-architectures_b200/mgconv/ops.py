@@ -114,6 +114,14 @@ class Combine:
                         C.byref(self.bn_x) if self.bn_x is not None else None, self.n, self.arr,
                         C.byref(self.d), ptr(self.sums))
 
+    def run_frozen(self, bn, g, write_d):
+        """the same sum, for a tensor that feeds BatchNorm `bn` in evaluation mode: writes g = gamma * invstd_r * d (and d only
+        when write_d) and accumulates (sum d, sum d*y) into self.sums (mg_grad_combine_bn_frozen)"""
+        if self.noop:
+            return
+        self.E.ctx.call("mg_grad_combine_bn_frozen", C.byref(self.x), self.relu_mask, C.byref(self.bn_x), self.n, self.arr,
+                        ptr(bn.weight), ptr(bn.running_var), bn.eps, C.byref(g), C.byref(self.d) if write_d else None, ptr(self.sums))
+
 
 def plan_companion_grad(E, x, p):
     """route the gradient of p = maxpool2x2_ceil(x) into x (arg-max recomputed from x in the combine).
@@ -186,11 +194,13 @@ class InputOp(Op):
 
 
 class AvgPoolOp(Op):
-    """cudnn.SpatialAveragePooling(r,r,r,r) of the input image (ilsvrc/rnmg.lua:175-177)"""
+    """cudnn.SpatialAveragePooling(r,r,r,r) of the input image (ilsvrc/rnmg.lua:175-177); backward (needInputGrad): the gradient of
+    the pooled image spread over its r x r windows, one more gradient source of the image"""
 
     def __init__(self, inp, r, out):
         self.inp, self.r, self.out = inp, r, out
         out.producer = self
+        self.comb = None
 
     def setup_fwd(self, E):
         self.out.buf = E.alloc(self.out.shape())
@@ -200,10 +210,30 @@ class AvgPoolOp(Op):
         return _keys(self.inp.buf), _keys(self.out.buf)
 
     def io_bwd(self):
-        return [], []
+        if self.comb is None:
+            return [], []
+        return _merge(self.comb.io(), (_keys(self.comb.buf), _keys(self.din)))
 
     def fwd(self, E):
         E.ctx.call("mg_avgpool_forward", C.byref(self.gi), self.r, C.byref(self.go))
+
+    def setup_bwd(self, E):
+        if self.inp.needs_grad and self.out.needs_grad:
+            t = self.inp
+            self.comb = Combine(E, self.out)
+            self.din = E.alloc(t.shape())
+            self.dg_out, self.dg_in = self.comb.grid(), t.grid(self.din)
+            t.srcs.append(Src(self.din, t.H, t.W, t.C, t.Cp, 0, MG_SEG_SAME))
+
+    def bwd(self, E):
+        if self.comb is not None:
+            self.comb.run()
+            E.ctx.call("mg_avgpool_backward", C.byref(self.dg_out), self.r, C.byref(self.dg_in))
+
+
+def _stats(conv):
+    """BatchNorm sums a convolution's epilogue reduces: none when the BatchNorm that follows is frozen (it reads running statistics)"""
+    return None if conv.apply is not None and conv.apply.frozen else ptr(conv.sums)
 
 
 class ConvOp(Op):
@@ -326,7 +356,7 @@ class ConvOp(Op):
         if self.col is not None:
             E.ctx.call("mg_im2col", C.byref(self.in_g), self.k, self.stride, self.pad, C.byref(self.col_g))
         E.ctx.call("mg_conv_forward", C.byref(self.desc), ptr(self.mod.weight), ptr(self.wpack), ptr(self.mod.bias),
-                   C.byref(self.yg), ptr(self.sums))
+                   C.byref(self.yg), _stats(self))
 
     def setup_bwd(self, E):
         if self.apply is None:  # plain convolution (Linear head): gradient of y comes straight from its consumers
@@ -417,7 +447,7 @@ class UpConvOp(Op):
         return _merge(io, (_keys(self.y.G, self.inp.buf), _keys(self.mod.gradWeight, self.mod.gradBias, self.dx)))
 
     def fwd(self, E):
-        E.ctx.call("mg_upconv2x2_forward", C.byref(self.gi), ptr(self.mod.weight), ptr(self.mod.bias), C.byref(self.yg), ptr(self.sums))
+        E.ctx.call("mg_upconv2x2_forward", C.byref(self.gi), ptr(self.mod.weight), ptr(self.mod.bias), C.byref(self.yg), _stats(self))
 
     def setup_bwd(self, E):
         if self.apply is None:
@@ -451,6 +481,9 @@ class ApplyOp(Op):
         out.producer = self
         self.pooled = None
         self.pool3 = None    # Pool3Op fused into this pass (fuse_stem_pool3): BN + ReLU + 3x3 / stride-2 max-pool, `out` never stored
+        # the BatchNorm runs in evaluation mode (running statistics, no update; backward through the frozen affine): set by the
+        # engine before every forward from the model's mode and the module's own train flag (Engine.forward)
+        self.frozen = False
 
     def setup_fwd(self, E):
         t, y = self.out, self.conv.y
@@ -473,15 +506,16 @@ class ApplyOp(Op):
 
     def _bn_struct(self, E):
         bn = self.bn
+        training = not self.frozen
         key = (bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
-               bool(E.training), E.bn_sync, float(bn.eps), float(bn.momentum))
+               training, E.bn_sync, float(bn.eps), float(bn.momentum))
         if self.bnf is None or self.bnf_key != key:
             f = mg_bn_fused()
             f.sums = self.conv.sums.data_ptr()
-            f.count = self.count * (max(1, E.bn_sync) if E.training else 1)
+            f.count = self.count * (max(1, E.bn_sync) if training else 1)
             f.gamma, f.beta = bn.weight.data_ptr(), bn.bias.data_ptr()
             f.running_mean, f.running_var = bn.running_mean.data_ptr(), bn.running_var.data_ptr()
-            f.eps, f.momentum, f.training = bn.eps, bn.momentum, int(E.training)
+            f.eps, f.momentum, f.training = bn.eps, bn.momentum, int(training)
             f.save_mean, f.save_invstd = self.mean.data_ptr(), self.invstd.data_ptr()
             self.bnf, self.bnf_key = f, key
         return self.bnf
@@ -509,7 +543,7 @@ class ApplyOp(Op):
         rg = C.byref(self.rg) if self.rg is not None else None
         pg = C.byref(self.pg) if self.pg is not None else None
         if bn is not None:
-            if E.bn_sync and E.training and not synced:   # cross-replica statistics: sum (sum y, sum y^2) over the ranks
+            if E.bn_sync and not self.frozen and not synced:   # cross-replica statistics: sum (sum y, sum y^2) over the ranks
                 E.ctx.call("mg_allreduce_inline", ptr(self.conv.sums), self.conv.sums.numel(), 2)   # int64 limbs of mg_sum
             if self.pool3 is not None:   # stem: + SpatialMaxPooling(3,3,2,2,1,1), arg-max codes for the backward routing
                 E.ctx.call("mg_bn_relu_pool3_forward", C.byref(self.zg), C.byref(self._bn_struct(E)), C.byref(self.pool3.go), ptr(self.pool3.code))
@@ -528,6 +562,8 @@ class ApplyOp(Op):
         D = self.comb.buf
         if self.res is not None and self.res.needs_grad:
             self.res.srcs.append(Src(D, t.H, t.W, t.C, t.Cp, 0, MG_SEG_SAME))
+        # frozen BatchNorm: the combine writes G itself, and D only when the shortcut reads it
+        self.d_for_res = self.res is not None and self.res.needs_grad
         if self.bn is not None:
             G = E.alloc(t.shape()) if self.res is not None else D   # the shortcut still reads D
             self.G = G   # keep the storage alive: the mg_grid structs below only hold raw pointers
@@ -545,11 +581,20 @@ class ApplyOp(Op):
     def bwd_combine(self, E):
         if self.pc is not None:
             self.pc.run()
-        self.comb.run()
+        if self.frozen:
+            self.comb.run_frozen(self.bn, self.gg, self.d_for_res)
+        else:
+            self.comb.run()
 
     def bwd_bn(self, E, synced=False):
         bn = self.bn
-        if bn is not None:
+        if bn is not None and self.frozen:
+            # the sums are this rank's own: every rank adds its full share of dgamma / dbeta / gradBias, the gradient all-reduce
+            # sums them like any other parameter gradient
+            E.ctx.call("mg_bn_backward_frozen", ptr(self.dsums), self.out.C, ptr(bn.weight), ptr(bn.running_mean), ptr(bn.running_var),
+                       bn.eps, ptr(bn.gradWeight), ptr(bn.gradBias), E.gscale, ptr(self.conv.mod.gradBias))
+            E.param_done(bn)
+        elif bn is not None:
             if E.bn_sync and not synced:
                 E.ctx.call("mg_allreduce_inline", ptr(self.dsums), self.dsums.numel(), 2)
             E.ctx.call("mg_bn_backward", C.byref(self.yraw), C.byref(self.dg), C.byref(self.gg), ptr(self.dsums), self.count * max(1, E.bn_sync),
