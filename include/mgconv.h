@@ -300,6 +300,29 @@ int mg_grad_combine_bn_frozen(mg_ctx* ctx, const mg_grid* x, int relu_mask, cons
                               const float* gamma, const float* running_var, float eps, mg_grid* g, mg_grid* d, mg_sum* bn_sums);
 int mg_bn_backward_frozen(mg_ctx* ctx, const mg_sum* bn_sums, int32_t C, const float* gamma, const float* running_mean,
                           const float* running_var, float eps, float* dgamma, float* dbeta, float gscale, float* conv_dbias);
+/* accGradParameters of n BatchNorm layers in one launch (up to 128 layers per launch; more take several).  The backward is
+ * then split in two: the updateGradInput phase calls mg_bn_backward (or mg_grad_combine_bn_frozen) with dgamma, dbeta and
+ * conv_dbias NULL, leaves the sums (sum d, sum d*y) it reduced in place, and this call turns them into the parameter
+ * gradients.  A training job adds exactly what mg_bn_backward adds with the same arguments (grids of Cp = padded C); a frozen
+ * job exactly what mg_bn_backward_frozen adds: the expressions are shared, the bits equal.  No floating-point atomics: a
+ * layer must not appear twice in one call. */
+typedef struct {
+  const mg_sum* sums;       /* [2*C] (sum d, sum d*y) of the layer's backward */
+  int64_t count;            /* training: elements per channel, as given to mg_bn_backward */
+  int32_t C;
+  int32_t frozen;           /* 0: training mode (save_mean / save_invstd), 1: evaluation mode (running statistics, eps) */
+  const float* gamma;       /* nullable: 1 */
+  const float* save_mean;   /* training */
+  const float* save_invstd;
+  const float* running_mean;   /* frozen */
+  const float* running_var;
+  float eps;
+  float gscale;
+  float* dgamma;            /* each nullable; += */
+  float* dbeta;
+  float* conv_dbias;
+} mg_bn_param_job;
+int mg_bn_param_grad(mg_ctx* ctx, int32_t n, const mg_bn_param_job* jobs);
 /* dcat = conv_transpose(g, w): gradient w.r.t. the concatenated input, segment s at channel
  * offset sum_{t<s} Cp_t.  Strided descriptors (the image-fed stem cudnn.SpatialConvolution(3, C, 7,7, 2,2, 3,3), rnmg.lua:180:
  * one unresampled segment of at most 8 channels) run a CUDA-core kernel from the fp32 weights w in both dtypes; wpack_t is unused. */
@@ -346,6 +369,16 @@ int mg_stage_forward(mg_stage_plan* plan, void* workspace, const float* const* x
  * differentiated in evaluation mode (running statistics, mg_grad_combine_bn_frozen / mg_bn_backward_frozen); after training != 0
  * in training mode (batch statistics, mg_bn_backward).  Calling it before any mg_stage_forward is an error. */
 int mg_stage_backward(mg_stage_plan* plan, void* workspace, const float* const* dy, const mg_stage_params* params, float* const* dx, float scale);
+/* The same backward in the two halves of the nn protocol:
+ *   mg_stage_forward -> mg_stage_update_grad_input -> mg_stage_acc_grad_parameters(scale) [-> mg_stage_acc_grad_parameters ...]
+ * mg_stage_update_grad_input: dy[i] -> dx[i] (as mg_stage_backward) and every internal gradient; writes no gradWeight / gradBias
+ * (params' gradient pointers may be NULL) and runs no weight-gradient kernel.  mg_stage_acc_grad_parameters: adds scale * the
+ * parameter gradients of the dy given to the last mg_stage_update_grad_input, from what that call left in the workspace (so
+ * the workspace must not be used by another call in between); a second call adds them again.  It is an error without an
+ * mg_stage_update_grad_input since the last mg_stage_forward.  Both follow the BatchNorm mode of the last mg_stage_forward, and
+ * the pair leaves the bits mg_stage_backward(scale) leaves. */
+int mg_stage_update_grad_input(mg_stage_plan* plan, void* workspace, const float* const* dy, const mg_stage_params* params, float* const* dx);
+int mg_stage_acc_grad_parameters(mg_stage_plan* plan, void* workspace, const mg_stage_params* params, float scale);
 
 /* ---- head / criterion / optimiser ("next" rows of the scope table) ------------------- */
 /* LogSoftMax + ClassNLLCriterion (mean): logits grid N x 1 x 1 x C; target int32 0-based;

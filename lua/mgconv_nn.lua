@@ -186,8 +186,25 @@ function MGStage:backward(input, gradOutput, scale)
                                      ptr_array(self.gradInput, n), scale or 1))
    return self.gradInput
 end
-function MGStage:updateGradInput(input, gradOutput) return self:backward(input, gradOutput, 0) end
-function MGStage:accGradParameters() end   -- done by backward()
+
+-- the two halves on their own (nngraph's gModule, hand-written loops, input-gradient tools): updateGradInput computes gradInput
+-- and launches no weight-gradient kernel; accGradParameters adds scale * the parameter gradients of the gradOutput given to the
+-- last updateGradInput (what that call left in the workspace: gradOutput itself is not read again).  Calling accGradParameters
+-- without an updateGradInput since the last updateOutput is an error.
+function MGStage:updateGradInput(input, gradOutput)
+   local ctx, ws = self:_state(input)
+   local n = #self.nIPs
+   local dy = {}
+   for i = 1, n do dy[i] = gradOutput[i]:contiguous() end
+   mg.check(ctx, C.mg_stage_update_grad_input(self._plan, ws, ffi.cast('const float* const*', ptr_array(dy, n)), self:_params(),
+                                              ptr_array(self.gradInput, n)))
+   return self.gradInput
+end
+
+function MGStage:accGradParameters(input, gradOutput, scale)
+   local ctx, ws = self:_state(input)
+   mg.check(ctx, C.mg_stage_acc_grad_parameters(self._plan, ws, self:_params(), scale or 1))
+end
 
 function MGStage:zeroGradParameters()
    for k = 1, #self.convs do

@@ -272,6 +272,54 @@ __host__ __device__ __forceinline__ double mg_sum_get(const mg_sum& s) {
 __device__ __forceinline__ double frozen_bn_invstd(float rvar, float eps) { return 1.0 / sqrt((double)rvar + (double)eps); }
 struct FrozenBn { const float* gamma; const float* running_var; float eps; const mg_grid* g; };
 
+// Training-mode BatchNorm backward of one channel from the sums sd = sum d, sdx = sum d*y over n elements, the batch mean mu,
+// invstd `is` and gamma g: dg = is * (sdx - mu * sd) and the coefficients of G = A*d + B*y + C.  RECIP divides by n through
+// rn = 1 / n (the one-pass bf16 kernel: no fp64 division per CTA), else by n itself (the fp32 coefficient kernel).  Every
+// kernel that derives these terms (mg_bn_backward, mg_bn_backward_frozen, mg_bn_param_grad) goes through the functions below,
+// written operation by operation with the _rn intrinsics, which the compiler never contracts or reorders: the rounding of each
+// step is fixed by the source, not by how the surrounding kernel was scheduled, so the split backward adds exactly the bits of
+// the fused one.  (The steps are the ones nvcc made of the plain expressions these functions replace.)
+struct BnTrainTerms { double dg, Ad, Bd, Cd; };
+template <bool RECIP>
+__device__ __forceinline__ BnTrainTerms bn_train_terms(double sd, double sdx, double mu, double is, double g, double n, double rn) {
+  BnTrainTerms t;
+  t.dg = __dmul_rn(is, __fma_rn(mu, -sd, sdx));                  // is * (sdx - mu * sd)
+  t.Ad = __dmul_rn(g, is);
+  const double b = __dmul_rn(__dmul_rn(-t.Ad, is), t.dg);         // -g * is * is * dg
+  const double x = __dmul_rn(__dmul_rn(mu, is), t.dg);            // mu * is * dg
+  if (RECIP) {
+    t.Bd = __dmul_rn(b, rn);
+    t.Cd = __dmul_rn(t.Ad, __fma_rn(x, rn, -__dmul_rn(sd, rn)));  // g * is * (x / n - sd / n)
+  } else {
+    t.Bd = __ddiv_rn(b, n);
+    t.Cd = __dmul_rn(t.Ad, __dsub_rn(__ddiv_rn(x, n), __ddiv_rn(sd, n)));
+  }
+  return t;
+}
+// dgamma += gscale * dg, dbeta += gscale * sum d, and the gradBias of the convolution that produced y += gscale * sum over
+// pixels of G = A * sum d + B * sum y + C * n (identically zero in exact arithmetic: rounding noise in the reference as well)
+__device__ __forceinline__ void bn_train_param_grad(const BnTrainTerms& t, double sd, double mu, double n, int c, float* dgamma,
+                                                    float* dbeta, float* conv_dbias, float gscale) {
+  if (dgamma) dgamma[c] = __fmaf_rn((float)t.dg, gscale, dgamma[c]);
+  if (dbeta) dbeta[c] = __fmaf_rn((float)sd, gscale, dbeta[c]);
+  if (conv_dbias) {
+    const double s = __fma_rn(n, t.Cd, __fma_rn(t.Ad, sd, __dmul_rn(t.Bd, __dmul_rn(mu, n))));
+    conv_dbias[c] = __fmaf_rn((float)s, gscale, conv_dbias[c]);
+  }
+}
+// frozen BatchNorm: dgamma += gscale * invstd_r * (sum d*y - mu_r * sum d), dbeta += gscale * sum d and the producing
+// convolution's gradBias += gscale * A * sum d (= the pixel sum of G = A * d), A = gamma * invstd_r
+__device__ __forceinline__ void bn_frozen_param_grad(const mg_sum* sums, int C, int c, const float* gamma, const float* rmean,
+                                                     const float* rvar, float eps, float* dgamma, float* dbeta, float gscale,
+                                                     float* conv_dbias) {
+  const double sd = mg_sum_get(sums[c]), sdy = mg_sum_get(sums[C + c]);
+  const double is = frozen_bn_invstd(rvar[c], eps);
+  if (dgamma) dgamma[c] = __fmaf_rn((float)__dmul_rn(is, __fma_rn((double)rmean[c], -sd, sdy)), gscale, dgamma[c]);
+  if (dbeta) dbeta[c] = __fmaf_rn((float)sd, gscale, dbeta[c]);
+  const float A = (float)__dmul_rn(gamma ? (double)gamma[c] : 1.0, is);
+  if (conv_dbias) conv_dbias[c] = __fmaf_rn((float)__dmul_rn((double)A, sd), gscale, conv_dbias[c]);
+}
+
 // ---- programmatic dependent launch (PDL) ---------------------------------------------------------
 // A kernel launched with mg_launch_pdl may become resident while its predecessor in the stream is still
 // draining; it must execute pdl_wait() before touching anything the predecessor wrote.  pdl_launch() (first

@@ -347,19 +347,14 @@ __global__ void bn_bwd_coef_kernel(const mg_sum* sums, int64_t count, int C, int
   int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= Cp) return;
   if (c >= C) { coef[c] = 0.f; coef[Cp + c] = 0.f; coef[2 * Cp + c] = 0.f; return; }
-  double sd = mg_sum_get(sums[c]), sdx = mg_sum_get(sums[C + c]);
-  double mu = mean[c], is = invstd[c], g = gamma ? gamma[c] : 1.0;
-  double dg = is * (sdx - mu * sd);
-  if (dgamma) dgamma[c] += gscale * (float)dg;
-  if (dbeta) dbeta[c] += gscale * (float)sd;
-  double n = (double)count;
-  const double Ad = g * is, Bd = -g * is * is * dg / n, Cd = g * is * (mu * is * dg / n - sd / n);
-  coef[c] = (float)Ad;
-  coef[Cp + c] = (float)Bd;
-  coef[2 * Cp + c] = (float)Cd;
-  // gradBias of the convolution that produced xraw = sum over pixels of the result = A*sum d + B*sum xraw + C*n
-  // (identically zero in exact arithmetic: pure rounding noise in the reference as well)
-  if (conv_dbias) conv_dbias[c] += gscale * (float)(Ad * sd + Bd * (mu * n) + Cd * n);
+  const double sd = mg_sum_get(sums[c]), sdx = mg_sum_get(sums[C + c]);
+  const double mu = mean[c], is = invstd[c], g = gamma ? gamma[c] : 1.0;
+  const double n = (double)count;
+  const BnTrainTerms t = bn_train_terms<false>(sd, sdx, mu, is, g, n, 0.0);
+  coef[c] = (float)t.Ad;
+  coef[Cp + c] = (float)t.Bd;
+  coef[2 * Cp + c] = (float)t.Cd;
+  bn_train_param_grad(t, sd, mu, n, c, dgamma, dbeta, conv_dbias, gscale);
 }
 
 template <typename T>
@@ -383,12 +378,36 @@ __global__ void bn_bwd_frozen_kernel(const mg_sum* sums, int C, const float* gam
   pdl_wait();
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  const double sd = mg_sum_get(sums[c]), sdy = mg_sum_get(sums[C + c]);
-  const double is = frozen_bn_invstd(rvar[c], eps);
-  if (dgamma) dgamma[c] += gscale * (float)(is * (sdy - (double)rmean[c] * sd));
-  if (dbeta) dbeta[c] += gscale * (float)sd;
-  const float A = (float)((gamma ? (double)gamma[c] : 1.0) * is);
-  if (conv_dbias) conv_dbias[c] += gscale * (float)((double)A * sd);
+  bn_frozen_param_grad(sums, C, c, gamma, rmean, rvar, eps, dgamma, dbeta, gscale, conv_dbias);
+}
+
+// accGradParameters of many BatchNorm layers in one launch (mg_bn_param_grad): blockIdx.y = layer, one thread per channel.
+// Each layer takes the expressions of the backward it replaces -- the frozen kernel above, or bn_train_terms in the form the
+// fused training backward of this context uses for it (recip: the one-pass bf16 kernel) -- so the bits are those of backward.
+// The job table travels as the kernel's parameter block (12 KB, __grid_constant__): no upload, nothing but the launch is seen
+// by a CUDA-graph capture.  R-MG-34 has 75 BatchNorm layers: one launch.
+constexpr int MG_BN_PARAM_CHUNK = 128;
+struct BnParamBatch {
+  mg_bn_param_job job[MG_BN_PARAM_CHUNK];
+  uint8_t recip[MG_BN_PARAM_CHUNK];
+};
+
+__global__ void bn_param_grad_kernel(const __grid_constant__ BnParamBatch b) {
+  pdl_launch();
+  pdl_wait();
+  const mg_bn_param_job& j = b.job[blockIdx.y];
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= j.C) return;
+  if (j.frozen) {
+    bn_frozen_param_grad(j.sums, j.C, c, j.gamma, j.running_mean, j.running_var, j.eps, j.dgamma, j.dbeta, j.gscale, j.conv_dbias);
+    return;
+  }
+  const double sd = mg_sum_get(j.sums[c]), sdx = mg_sum_get(j.sums[j.C + c]);
+  const double mu = j.save_mean[c], is = j.save_invstd[c], g = j.gamma ? j.gamma[c] : 1.0;
+  const double n = (double)j.count;
+  const BnTrainTerms t = b.recip[blockIdx.y] ? bn_train_terms<true>(sd, sdx, mu, is, g, n, 1.0 / n)
+                                             : bn_train_terms<false>(sd, sdx, mu, is, g, n, 0.0);
+  bn_train_param_grad(t, sd, mu, n, c, j.dgamma, j.dbeta, j.conv_dbias, j.gscale);
 }
 
 // ---------------------------------------------------------------- input path: crop / flip / normalise ----------
@@ -840,6 +859,31 @@ int mg_bn_backward_frozen(mg_ctx* ctx, const mg_sum* bn_sums, int32_t C, const f
   mg_launch_pdl(bn_bwd_frozen_kernel, dim3((unsigned)mg_cdiv(C, 128)), dim3(128), 0, ctx->stream, bn_sums, (int)C, gamma, running_mean, running_var,
                 eps, dgamma, dbeta, gscale, conv_dbias);
   MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
+}
+
+int mg_bn_param_grad(mg_ctx* ctx, int32_t n, const mg_bn_param_job* jobs) {
+  if (!ctx || n < 0 || (n && !jobs)) return MG_ERR_INVALID_ARG;
+  for (int32_t j0 = 0; j0 < n; j0 += MG_BN_PARAM_CHUNK) {
+    const int m = std::min<int>(MG_BN_PARAM_CHUNK, n - j0);
+    BnParamBatch b;
+    memset(&b, 0, sizeof(b));
+    int cmax = 0;
+    for (int k = 0; k < m; ++k) {
+      const mg_bn_param_job& j = jobs[j0 + k];
+      MG_REQUIRE(ctx, j.sums && j.C >= 1, MG_ERR_INVALID_ARG, "bn_param_grad: job %d has no sums or no channels", j0 + k);
+      if (j.frozen)
+        MG_REQUIRE(ctx, j.running_mean && j.running_var, MG_ERR_INVALID_ARG, "bn_param_grad: frozen job %d needs the running statistics", j0 + k);
+      else
+        MG_REQUIRE(ctx, j.save_mean && j.save_invstd && j.count >= 1, MG_ERR_INVALID_ARG, "bn_param_grad: job %d needs save_mean / save_invstd / count", j0 + k);
+      b.job[k] = j;
+      // the form mg_bn_backward takes for grids of Cp = padded C: bf16 one pass up to 2048 channels (bf16_bn_bwd_apply), else the coefficient kernel
+      b.recip[k] = ctx->dtype == MG_BF16 && (j.C + 7) / 8 * 8 <= 2048;
+      cmax = std::max(cmax, (int)j.C);
+    }
+    mg_launch_pdl(bn_param_grad_kernel, dim3((unsigned)mg_cdiv(cmax, 128), (unsigned)m), dim3(128), 0, ctx->stream, b);
+    MG_CHECK_LAUNCH(ctx);
+  }
   return MG_OK;
 }
 

@@ -650,15 +650,10 @@ __global__ void __launch_bounds__(256, 3) bn_bwd_apply_bf16_kernel(const bf16* _
     if (c < C) {
       const double sd = mg_sum_get(bp.sums[c]), sdx = mg_sum_get(bp.sums[C + c]);
       const double mu = bp.mean[c], is = bp.invstd[c], g = bp.gamma ? bp.gamma[c] : 1.0;
-      const double dg = is * (sdx - mu * sd);
       const double n = (double)bp.count, rn = bp.inv_count;   // reciprocal from the host: no fp64 division routine per CTA
-      const double Ad = g * is, Bd = -g * is * is * dg * rn, Cd = g * is * (mu * is * dg * rn - sd * rn);
-      if (blockIdx.x == 0) {
-        if (bp.dgamma) bp.dgamma[c] += gscale * (float)dg;
-        if (bp.dbeta) bp.dbeta[c] += gscale * (float)sd;
-        if (dbias) dbias[c] += gscale * (float)(Ad * sd + Bd * (mu * n) + Cd * n);
-      }
-      A = (float)Ad; B = (float)Bd; Cc = (float)Cd;
+      const BnTrainTerms t = bn_train_terms<true>(sd, sdx, mu, is, g, n, rn);
+      if (blockIdx.x == 0) bn_train_param_grad(t, sd, mu, n, c, bp.dgamma, bp.dbeta, dbias, gscale);
+      A = (float)t.Ad; B = (float)t.Bd; Cc = (float)t.Cd;
     }
     s_coef[c] = A; s_coef[V * 8 + c] = B; s_coef[2 * V * 8 + c] = Cc;
   }

@@ -16,6 +16,7 @@ struct mg_stage_plan {
   mg_stage_desc d;
   int batch, n, layers, elt;
   int last_training;   // training flag of the last mg_stage_forward (-1: none yet); mg_stage_backward differentiates that mode
+  int grad_input_ready;   // mg_stage_update_grad_input ran since the last mg_stage_forward: mg_stage_acc_grad_parameters may follow
   // byte offsets into the workspace
   size_t X[MG_STAGE_MAX_GRIDS], PX[MG_STAGE_MAX_GRIDS], DX[MG_STAGE_MAX_GRIDS], DY[MG_STAGE_MAX_GRIDS];
   size_t y[2][MG_STAGE_MAX_GRIDS], a[2][MG_STAGE_MAX_GRIDS], Pa[2][MG_STAGE_MAX_GRIDS];
@@ -152,6 +153,7 @@ int mg_stage_forward(mg_stage_plan* p, void* workspace, const float* const* x, c
   MG_REQUIRE(ctx, ((uintptr_t)workspace & 255) == 0, MG_ERR_INVALID_ARG, "stage_forward: workspace must be 256-byte aligned");
   MG_TRY(mg_memset_zero(ctx, ws + p->sums_begin, p->sums_bytes));
   p->last_training = training ? 1 : 0;
+  p->grad_input_ready = 0;
   // inputs: NCHW fp32 -> grids, plus the pooled companion every coarser neighbour gathers
   for (int i = 0; i < n; ++i) {
     MG_REQUIRE(ctx, x[i] != nullptr, MG_ERR_INVALID_ARG, "stage_forward: x[%d] is null", i);
@@ -200,13 +202,21 @@ int mg_stage_forward(mg_stage_plan* p, void* workspace, const float* const* x, c
   return MG_OK;
 }
 
-int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy, const mg_stage_params* prm, float* const* dx, float scale) {
+}  // extern "C"
+
+namespace {
+
+// mg_stage_backward (params: every gradient) and mg_stage_update_grad_input (!params: the data gradient alone -- BatchNorm
+// with dgamma / dbeta / conv_dbias NULL, no weight gradient; the sums of every layer stay in the workspace for
+// mg_stage_acc_grad_parameters)
+int stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy, const mg_stage_params* prm, float* const* dx, float scale,
+                   bool params, const char* who) {
   if (!p || !workspace || !dy || !prm) return MG_ERR_INVALID_ARG;
   mg_ctx* ctx = p->ctx;
   const mg_stage_desc& d = p->d;
   const int n = p->n, L = p->layers, B = p->batch;
   char* ws = (char*)workspace;
-  MG_REQUIRE(ctx, p->last_training >= 0, MG_ERR_INVALID_ARG, "stage_backward: no mg_stage_forward on this plan yet");
+  MG_REQUIRE(ctx, p->last_training >= 0, MG_ERR_INVALID_ARG, "%s: no mg_stage_forward on this plan yet", who);
   const bool frozen = p->last_training == 0;
   for (int i = 0; i < n; ++i) {
     MG_REQUIRE(ctx, dy[i] != nullptr, MG_ERR_INVALID_ARG, "stage_backward: dy[%d] is null", i);
@@ -217,8 +227,12 @@ int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy,
     const bool last = l + 1 == L;
     for (int i = 0; i < n; ++i) {
       const int k = l * n + i;
-      MG_REQUIRE(ctx, prm->conv_gw[k] && prm->conv_gb[k] && prm->bn_gg[k] && prm->bn_gb[k], MG_ERR_INVALID_ARG,
-                 "stage_backward: gradient tensors of conv / BN %d are null", k);
+      if (params)
+        MG_REQUIRE(ctx, prm->conv_gw[k] && prm->conv_gb[k] && prm->bn_gg[k] && prm->bn_gb[k], MG_ERR_INVALID_ARG,
+                   "%s: gradient tensors of conv / BN %d are null", who, k);
+      float* const bn_gg = params ? prm->bn_gg[k] : nullptr;
+      float* const bn_gb = params ? prm->bn_gb[k] : nullptr;
+      float* const conv_gb = params ? prm->conv_gb[k] : nullptr;
       // gradient of a_l,i in gather form: its consumers' contributions, times its ReLU mask, plus the BN sums
       mg_grad_src src[3];
       int ns = 0;
@@ -249,16 +263,16 @@ int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy,
       const int relu = last ? (d.no_final_relu ? 0 : 1) : 1;
       if (frozen) {   // evaluation-mode BatchNorm: G = gamma * invstd_r * D in the combine pass; D itself only for the shortcut
         MG_TRY(mg_grad_combine_bn_frozen(ctx, &A, relu, &Yraw, ns, src, prm->bn_g[k], prm->bn_rv[k], d.eps, &Gg, (last && d.residual) ? &Dg : nullptr, bs));
-        MG_TRY(mg_bn_backward_frozen(ctx, bs, d.C_out[i], prm->bn_g[k], prm->bn_rm[k], prm->bn_rv[k], d.eps, prm->bn_gg[k], prm->bn_gb[k], scale,
-                                     prm->conv_gb[k]));
+        if (params)
+          MG_TRY(mg_bn_backward_frozen(ctx, bs, d.C_out[i], prm->bn_g[k], prm->bn_rm[k], prm->bn_rv[k], d.eps, bn_gg, bn_gb, scale, conv_gb));
       } else {
         MG_TRY(mg_grad_combine(ctx, &A, relu, &Yraw, ns, src, &Dg, bs));
         MG_TRY(mg_bn_backward(ctx, &Yraw, &Dg, &Gg, bs, (int64_t)B * d.H[i] * d.W[i], prm->bn_g[k], (const float*)(ws + p->mean[l][i]),
-                              (const float*)(ws + p->invstd[l][i]), prm->bn_gg[k], prm->bn_gb[k], scale, (float*)(ws + p->coef[l][i]), prm->conv_gb[k]));
+                              (const float*)(ws + p->invstd[l][i]), bn_gg, bn_gb, scale, (float*)(ws + p->coef[l][i]), conv_gb));
       }
       mg_conv_desc cd;
       make_desc(p, ws, l, i, &cd);
-      MG_TRY(mg_conv_backward_weight(ctx, &cd, &Gg, prm->conv_gw[k], nullptr, scale));
+      if (params) MG_TRY(mg_conv_backward_weight(ctx, &cd, &Gg, prm->conv_gw[k], nullptr, scale));
       void* wpt = p->wpack_t[l][i] == (size_t)-1 ? nullptr : ws + p->wpack_t[l][i];
       if (wpt) MG_TRY(mg_conv_pack_weights(ctx, &cd, prm->conv_w[k], wpt, 1));
       mg_grid DC = grid_of(ws, p->dcat[l][i], B, d.H[i], d.W[i], p->ccatp[l][i]);
@@ -294,6 +308,60 @@ int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy,
     MG_TRY(mg_grad_combine(ctx, &X, 0, nullptr, ns, src, &DX, nullptr));
     MG_TRY(mg_export_nchw(ctx, &DX, dx[i]));
   }
+  return MG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int mg_stage_backward(mg_stage_plan* p, void* workspace, const float* const* dy, const mg_stage_params* prm, float* const* dx, float scale) {
+  return stage_backward(p, workspace, dy, prm, dx, scale, true, "stage_backward");
+}
+
+int mg_stage_update_grad_input(mg_stage_plan* p, void* workspace, const float* const* dy, const mg_stage_params* prm, float* const* dx) {
+  const int rc = stage_backward(p, workspace, dy, prm, dx, 0.f, false, "stage_update_grad_input");
+  if (rc == MG_OK) p->grad_input_ready = 1;
+  return rc;
+}
+
+int mg_stage_acc_grad_parameters(mg_stage_plan* p, void* workspace, const mg_stage_params* prm, float scale) {
+  if (!p || !workspace || !prm) return MG_ERR_INVALID_ARG;
+  mg_ctx* ctx = p->ctx;
+  const mg_stage_desc& d = p->d;
+  const int n = p->n, L = p->layers, B = p->batch;
+  char* ws = (char*)workspace;
+  MG_REQUIRE(ctx, p->grad_input_ready, MG_ERR_INVALID_ARG,
+             "stage_acc_grad_parameters: no mg_stage_update_grad_input since the last mg_stage_forward of this plan");
+  const bool frozen = p->last_training == 0;
+  // every BatchNorm of the stage in one launch, from the sums, batch statistics and G the update phase left in the workspace
+  mg_bn_param_job jobs[2 * MG_STAGE_MAX_GRIDS];
+  memset(jobs, 0, sizeof(jobs));
+  for (int l = 0; l < L; ++l)
+    for (int i = 0; i < n; ++i) {
+      const int k = l * n + i;
+      MG_REQUIRE(ctx, prm->conv_gw[k] && prm->conv_gb[k] && prm->bn_gg[k] && prm->bn_gb[k], MG_ERR_INVALID_ARG,
+                 "stage_acc_grad_parameters: gradient tensors of conv / BN %d are null", k);
+      mg_bn_param_job& j = jobs[k];
+      j.sums = (const mg_sum*)(ws + p->bsums[l][i]);
+      j.count = (int64_t)B * d.H[i] * d.W[i];
+      j.C = d.C_out[i];
+      j.frozen = frozen ? 1 : 0;
+      j.gamma = prm->bn_g[k];
+      j.save_mean = (const float*)(ws + p->mean[l][i]); j.save_invstd = (const float*)(ws + p->invstd[l][i]);
+      j.running_mean = prm->bn_rm[k]; j.running_var = prm->bn_rv[k];
+      j.eps = d.eps;
+      j.gscale = scale;
+      j.dgamma = prm->bn_gg[k]; j.dbeta = prm->bn_gb[k]; j.conv_dbias = prm->conv_gb[k];
+    }
+  MG_TRY(mg_bn_param_grad(ctx, L * n, jobs));
+  for (int l = L - 1; l >= 0; --l)
+    for (int i = 0; i < n; ++i) {
+      mg_conv_desc cd;
+      make_desc(p, ws, l, i, &cd);
+      mg_grid Gg = grid_of(ws, p->G[l][i], B, d.H[i], d.W[i], d.C_out[i]);
+      MG_TRY(mg_conv_backward_weight(ctx, &cd, &Gg, prm->conv_gw[l * n + i], nullptr, scale));
+    }
   return MG_OK;
 }
 

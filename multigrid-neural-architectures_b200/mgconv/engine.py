@@ -82,7 +82,13 @@ class Engine:
         self._tuned_fwd = self._tuned_bwd = False
         # per-scale chains of a stage on separate CUDA streams (sched.py); MGCONV_LANES=1 runs the serial plan
         self.n_lanes = max(1, min(4, int(os.environ.get("MGCONV_LANES", "3"))))
-        self._sched_fwd = self._sched_bwd = None
+        self._sched_fwd = self._sched_bwd = self._sched_upd = self._sched_acc = None
+        self._acc_units = None
+        # split backward (updateGradInput / accGradParameters): forwards run so far, and the forward the last update_grad_input
+        # differentiated -- acc_grad_parameters reads what that call left in the plan's buffers
+        self.generation = 0
+        self.grad_input_generation = None
+        self._bn_jobs = None
         for m in model.listModules():
             for _, w, _ in m.own_parameters():
                 if w.device != self.device:
@@ -171,7 +177,8 @@ class Engine:
 
     def invalidate_schedules(self):
         """buffer addresses the schedules were derived from changed (parameters re-homed by getParameters())"""
-        self._sched_fwd = self._sched_bwd = None
+        self._sched_fwd = self._sched_bwd = self._sched_upd = self._sched_acc = None
+        self._acc_units = None
 
     def _bind_stream(self):
         self.ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
@@ -197,6 +204,7 @@ class Engine:
     def forward(self, input, training=True):
         self._bind_stream()
         self.training = training
+        self.generation += 1
         # a BatchNorm trains only when the model trains and its own module does (Torch7: bn:evaluate() inside model:training());
         # a frozen one normalises with its running statistics, leaves them alone, and is differentiated as that fixed affine
         for o in self.bn_ops:
@@ -237,12 +245,13 @@ class Engine:
         self.ctx.call("mg_allreduce_inline", C.c_void_p(lo), (hi - lo) // 8, 2)
         return True
 
-    def _run_sync_bn(self, oplist, fwd):
+    def _run_sync_bn(self, oplist, fwd, params=True):
+        """params = False: the backward of update_grad_input (no parameter gradients)"""
         i, n = 0, len(oplist)
         while i < n:
             o = oplist[i]
             if not isinstance(o, ops.ApplyOp):
-                (o.fwd if fwd else o.bwd)(self)
+                (o.fwd if fwd else o.bwd if params else o.bwd_input)(self)
                 i += 1
                 continue
             j = i
@@ -258,7 +267,7 @@ class Engine:
                     a.bwd_combine(self)
                 synced = self._allreduce_sums([a.dsums for a in run if a.bn is not None and not a.frozen])
                 for a in run:
-                    a.bwd_bn(self, synced=synced)
+                    a.bwd_bn(self, synced=synced, params=params)
             i = j
 
     def _results(self, s):
@@ -271,12 +280,11 @@ class Engine:
             o.setup_bwd(self)
         self._bwd_ready = True
 
-    def backward(self, gradOutput, scale=1.0):
+    def _begin_backward(self, gradOutput):
         self._bind_stream()
         if not self._bwd_ready:
             self._setup_bwd()
             self.pack_weights()  # transposed images for dgrad were allocated just now
-        self.gscale = float(scale)
         for op, g in zip(_flatten(self.out_struct), _flatten(gradOutput)):
             op.grad_out = g.contiguous().float()
         if self.autotune and not self._tuned_bwd and self.use_packed and not torch.cuda.is_current_stream_capturing():
@@ -285,6 +293,17 @@ class Engine:
                 o.tune_bwd(self)
             self._report_tuning("algo_bwd_data")
         self.zero_sums("bwd")
+
+    def _grad_input(self):
+        gi = [op.grad_nchw for op in self.input_ops]
+        if all(g is None for g in gi):
+            return None
+        return gi if len(gi) > 1 else gi[0]
+
+    def backward(self, gradOutput, scale=1.0):
+        self.gscale = float(scale)
+        self._begin_backward(gradOutput)
+        self.grad_input_generation = None   # the buffers now hold this backward's gradient
         if self._use_lanes():
             if self._sched_bwd is None:
                 # a convolution's backward is two units: dgrad (the next stage waits for it) on the lane of its scale,
@@ -304,7 +323,52 @@ class Engine:
         else:
             for o in reversed(self.plan.ops):
                 o.bwd(self)
-        gi = [op.grad_nchw for op in self.input_ops]
-        if all(g is None for g in gi):
-            return None
-        return gi if len(gi) > 1 else gi[0]
+        return self._grad_input()
+
+    # ---- backward in the two phases of the nn protocol --------------------------------------------------------------
+    # update_grad_input runs everything backward() runs except the parameter gradients: the data gradients, the dgrad half of
+    # every convolution, BatchNorm with no dgamma / dbeta / gradBias output.  The BatchNorm sums (the "bwd" arena) and every
+    # gradient grid stay where they are, and acc_grad_parameters turns them into the parameter gradients: one batched BatchNorm
+    # launch (mg_bn_param_grad), then the wgrad half of every convolution.  Each buffer gets the same writes in the same order
+    # as in backward(), so the pair leaves backward's bits.
+    def update_grad_input(self, gradOutput):
+        self._begin_backward(gradOutput)
+        if self._use_lanes():
+            if self._sched_upd is None:
+                units = [sched.Unit(o.io_bwd_input(), o.bwd_input, o.size()) for o in reversed(self.plan.ops)]
+                self._sched_upd = sched.Schedule(units, lambda u: u.io, lambda u: u.run, self.n_lanes, len(self.plan.ops) + 16)
+            self._sched_upd.run(self)
+        elif self.bn_sync:
+            # the data gradient needs the global (sum d, sum d*y): the all-reduce of the sums belongs to this phase
+            self._run_sync_bn(list(reversed(self.plan.ops)), fwd=False, params=False)
+        else:
+            for o in reversed(self.plan.ops):
+                o.bwd_input(self)
+        self.grad_input_generation = self.generation
+        return self._grad_input()
+
+    def acc_grad_parameters(self, scale=1.0):
+        if self.grad_input_generation != self.generation:
+            raise ffi.MGError("accGradParameters: no updateGradInput since the last forward -- it adds the parameter gradients "
+                              "of the gradOutput given to the last updateGradInput of the current forward")
+        self._bind_stream()
+        self.gscale = float(scale)
+        if self.bn_ops:
+            n = len(self.bn_ops)
+            if self._bn_jobs is None:
+                self._bn_jobs = (ffi.mg_bn_param_job * n)()
+            for o, j in zip(self.bn_ops, self._bn_jobs):
+                o.param_job(self, j)
+            self.ctx.call("mg_bn_param_grad", n, self._bn_jobs)
+            for o in self.bn_ops:
+                self.param_done(o.bn)
+        if self._acc_units is None:
+            self._acc_units = [sched.Unit(io, run, o.size()) for o in reversed(self.plan.ops) for io, run in o.acc_units()]
+        if self._use_lanes():
+            # the schedule starts behind everything on lane 0 (the update phase joined its lanes there, then the BatchNorm launch)
+            if self._sched_acc is None:
+                self._sched_acc = sched.Schedule(self._acc_units, lambda u: u.io, lambda u: u.run, self.n_lanes, len(self.plan.ops) + 16)
+            self._sched_acc.run(self)
+        else:
+            for u in self._acc_units:
+                u.run(self)

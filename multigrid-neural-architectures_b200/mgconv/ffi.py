@@ -60,6 +60,12 @@ class mg_bn_fused(C.Structure):
                 ("training", C.c_int32), ("save_mean", C.c_void_p), ("save_invstd", C.c_void_p)]
 
 
+class mg_bn_param_job(C.Structure):
+    _fields_ = [("sums", C.c_void_p), ("count", C.c_int64), ("C", C.c_int32), ("frozen", C.c_int32), ("gamma", C.c_void_p),
+                ("save_mean", C.c_void_p), ("save_invstd", C.c_void_p), ("running_mean", C.c_void_p), ("running_var", C.c_void_p),
+                ("eps", C.c_float), ("gscale", C.c_float), ("dgamma", C.c_void_p), ("dbeta", C.c_void_p), ("conv_dbias", C.c_void_p)]
+
+
 class mg_dropout(C.Structure):
     _fields_ = [("p", C.c_float), ("op", C.c_uint32), ("rank", C.c_uint32), ("seed", C.c_uint64), ("step", C.c_void_p)]
 
@@ -125,6 +131,7 @@ SIGNATURES = {
     "mg_bn_backward": (_I, [_P, _G, _G, _G, _P, _I64, _P, _P, _P, _P, _P, _F, _P, _P]),
     "mg_grad_combine_bn_frozen": (_I, [_P, _G, _I, _G, C.c_int32, C.POINTER(mg_grad_src), _P, _P, _F, _G, _G, _P]),
     "mg_bn_backward_frozen": (_I, [_P, _P, C.c_int32, _P, _P, _P, _F, _P, _P, _F, _P]),
+    "mg_bn_param_grad": (_I, [_P, C.c_int32, C.POINTER(mg_bn_param_job)]),
     "mg_conv_backward_data": (_I, [_P, _D, _P, _P, _G, _G]),
     "mg_conv_backward_weight": (_I, [_P, _D, _G, _P, _P, _F]),
     "mg_nll_forward_backward": (_I, [_P, _G, _P, _P, _P, _G, _F]),
@@ -141,6 +148,8 @@ SIGNATURES = {
     "mg_plan_destroy": (_I, [_P]),
     "mg_stage_forward": (_I, [_P, _P, C.POINTER(_P), C.POINTER(mg_stage_params), C.POINTER(_P), _I]),
     "mg_stage_backward": (_I, [_P, _P, C.POINTER(_P), C.POINTER(mg_stage_params), C.POINTER(_P), _F]),
+    "mg_stage_update_grad_input": (_I, [_P, _P, C.POINTER(_P), C.POINTER(mg_stage_params), C.POINTER(_P)]),
+    "mg_stage_acc_grad_parameters": (_I, [_P, _P, C.POINTER(mg_stage_params), _F]),
     "mg_comm_unique_id": (_I, [_P]),
     "mg_comm_init": (_I, [_P, _I, _I, _P]),
     "mg_comm_destroy": (_I, [_P]),

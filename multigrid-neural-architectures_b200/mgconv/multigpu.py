@@ -213,6 +213,23 @@ class DataParallel:
         eng = self.model._engine if input is None else self.model._get_engine(input)
         if self.world == 1 or self.gflat is None:
             return self.model.backward(input, gradOutput, scale)
+        return self._reduced(eng, lambda lb, gb: self.model.backward(input, gradOutput, scale * lb / gb))
+
+    def updateGradInput(self, input, gradOutput):
+        """the local data gradient: no parameter gradient is written, so nothing is all-reduced (-bnSync's all-reduce of the
+        BatchNorm sums is part of it: the data gradient needs the global sums)"""
+        return self.model.updateGradInput(input, gradOutput)
+
+    def accGradParameters(self, input, gradOutput=None, scale=1.0):
+        """backward's parameter half: the same shard weight and -iterSize stash, buckets all-reduced as they complete"""
+        eng = self.model._acc_engine(gradOutput)   # misuse raises before gflat is touched
+        if self.world == 1 or self.gflat is None:
+            return self.model.accGradParameters(input, gradOutput, scale)
+        self._reduced(eng, lambda lb, gb: eng.acc_grad_parameters(scale * lb / gb))
+
+    def _reduced(self, eng, run):
+        """run(local_B, global_B) adds this rank's parameter gradients, reporting each module through _param_done; every bucket is
+        all-reduced as soon as its last gradient was enqueued, the rest after run() returns"""
         self._reset_buckets()
         # Gradient accumulation (-iterSize, model.lua:39-44; pipelines/standard/train.lua:147-169 zeroes the gradients only
         # before the first micro-batch): backward ACCUMULATES into gflat, so all-reducing gflat in place would sum the
@@ -226,7 +243,7 @@ class DataParallel:
             self._gprev.copy_(self.gflat)
             self.gflat.zero_()
         local_B, global_B = getattr(eng, "shard", (1, self.world))
-        gi = self.model.backward(input, gradOutput, scale * local_B / global_B)
+        gi = run(local_B, global_B)
         for b, (off, cnt, _) in enumerate(self.buckets):   # parameters the plan never touched
             if b not in self.launched:
                 eng.ctx.call("mg_allreduce_launch", ptr(self.gflat[off:off + cnt]), cnt, 0)

@@ -10,7 +10,8 @@ concatenated tensor: they become segment descriptors of the consuming convolutio
 the zero-padded shortcut and CAddTable become the conv's epilogue pass.
 
 Module protocol kept from Torch7 (SURVEY.md section 8b): forward(input), backward(input,
-gradOutput), parameters(), getParameters(), zeroGradParameters(), training(), evaluate(),
+gradOutput), updateGradInput(input, gradOutput), accGradParameters(input, gradOutput, scale),
+parameters(), getParameters(), zeroGradParameters(), training(), evaluate(),
 findModules(typename), listModules(), apply(fn), cuda(), clearState(); fields .output,
 .gradInput, .train.  Tensors at the boundary are torch CUDA tensors, NCHW fp32, as the
 reference's put2GPU leaves them (utils/utilfuncs.lua:3-30).
@@ -18,9 +19,17 @@ reference's put2GPU leaves them (utils/utilfuncs.lua:3-30).
 import math
 import torch
 
+from . import ffi
 from . import lower as L
 
 MAX_ENGINES = 3   # lowered plans (with their activation buffers) kept per top-level module, one per input shape
+
+
+def _tensor_signature(t):
+    """(storage address, shape) of a tensor or nested table of tensors: what identifies "the very tensor" of updateGradInput"""
+    if isinstance(t, (list, tuple)):
+        return tuple(_tensor_signature(e) for e in t)
+    return (t.data_ptr(), tuple(t.shape))
 
 
 # ------------------------------------------------------------------------------------
@@ -161,6 +170,36 @@ class Module:
         eng = self._engine if input is None else self._get_engine(input)
         self.gradInput = eng.backward(gradOutput, scale)
         return self.gradInput
+
+    # backward() = updateGradInput() + accGradParameters(), as in Torch7, for hosts that call the halves themselves (nngraph's
+    # gModule, hand-written loops, saliency maps and adversarial inputs that want the image gradient alone)
+    def updateGradInput(self, input, gradOutput):
+        """gradInput (the image gradient when needInputGrad is set) and every internal gradient of the last forward; writes no
+        parameter gradient and launches no weight-gradient kernel"""
+        eng = self._engine if input is None else self._get_engine(input)
+        if eng is None or eng.generation == 0:
+            raise ffi.MGError("updateGradInput: no forward since the plan was built (clearState / getParameters / cuda)")
+        self.gradInput = eng.update_grad_input(gradOutput)
+        self._grad_output_seen = _tensor_signature(gradOutput)
+        return self.gradInput
+
+    def accGradParameters(self, input, gradOutput=None, scale=1.0):
+        """gradParameters += scale * dL/dtheta for the gradOutput given to the last updateGradInput of the current forward (a
+        second call adds it again).  The values used are those updateGradInput recorded: gradOutput is not read, it may be None
+        or must be that very tensor (same storage and shape).  Raises when there was no updateGradInput since the last forward
+        or since the plan was rebuilt (clearState, getParameters); `input` is the forward's, as in Torch7, and not used."""
+        self._acc_engine(gradOutput).acc_grad_parameters(scale)
+
+    def _acc_engine(self, gradOutput):
+        """the engine an accGradParameters call adds from, after the misuse checks"""
+        eng = self._engine
+        if eng is None or eng.grad_input_generation != eng.generation:
+            raise ffi.MGError("accGradParameters: no updateGradInput since the last forward (or the plan was rebuilt by "
+                              "clearState / getParameters): it adds the gradient recorded by updateGradInput")
+        if gradOutput is not None and _tensor_signature(gradOutput) != getattr(self, "_grad_output_seen", None):
+            raise ffi.MGError("accGradParameters: gradOutput is not the tensor given to updateGradInput -- the gradient it adds is "
+                              "the one updateGradInput recorded; pass that tensor or None")
+        return eng
 
     # ---- symbolic trace ---------------------------------------------------------------
     def trace(self, x, b):

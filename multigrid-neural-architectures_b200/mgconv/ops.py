@@ -12,7 +12,7 @@ import os
 import torch
 
 from . import ffi
-from .ffi import mg_grid, mg_conv_desc, mg_grad_src, mg_bn_fused, mg_dropout, ptr, MG_SEG_SAME, MG_SEG_POOL, MG_SEG_UP, MG_SRC_POOL3, MG_MAX_SRC
+from .ffi import mg_grid, mg_conv_desc, mg_grad_src, mg_bn_fused, mg_bn_param_job, mg_dropout, ptr, MG_SEG_SAME, MG_SEG_POOL, MG_SEG_UP, MG_SRC_POOL3, MG_MAX_SRC
 
 
 def cpad(c):
@@ -148,6 +148,12 @@ class Op:
     def io_fwd(self): return None
     def io_bwd(self): return None
     def size(self): return getattr(getattr(self, "out", None), "H", 0)
+    # bwd() in the two phases of the nn protocol (Engine.update_grad_input / acc_grad_parameters): bwd_input computes the
+    # gradients of the data and writes no parameter gradient; acc_units are the parameter-gradient work as (io, run) pairs.
+    # BatchNorm layers take part through ApplyOp.param_job (one batched launch of the engine) instead.
+    def bwd_input(self, E): self.bwd(E)
+    def io_bwd_input(self): return self.io_bwd()
+    def acc_units(self): return []
 
 
 def _merge(*ios):
@@ -395,6 +401,16 @@ class ConvOp(Op):
         self.bwd_data(E)
         self.bwd_weight(E)
 
+    def bwd_input(self, E):
+        self.bwd_data(E)
+
+    def io_bwd_input(self):
+        return self.bwd_units()[0][0]
+
+    def acc_units(self):
+        io_w, run, _ = self.bwd_units()[1]
+        return [(io_w, run)]
+
     def bwd_units(self):
         """the two independently schedulable halves of bwd() for the lane scheduler: (io, run, fixed lane or None)"""
         io_d = _merge(self.ycomb.io() if self.ycomb is not None else None,
@@ -467,6 +483,23 @@ class UpConvOp(Op):
                    C.byref(self.dxg) if self.dx is not None else None, ptr(self.mod.gradWeight),
                    None if fused_bias else ptr(self.mod.gradBias), E.gscale)
         E.param_done(self.mod)
+
+    def bwd_input(self, E):
+        """the dx half of mg_upconv2x2_backward (dw, dbias NULL)"""
+        if self.ycomb is not None:
+            self.ycomb.run()
+        if self.dx is not None:
+            E.ctx.call("mg_upconv2x2_backward", C.byref(self.gi), ptr(self.mod.weight), C.byref(self.y.G), C.byref(self.dxg), None, None, E.gscale)
+
+    def bwd_param(self, E):
+        """the dw / dbias half (dx NULL)"""
+        fused_bias = self.apply is not None and self.apply.bn is not None
+        E.ctx.call("mg_upconv2x2_backward", C.byref(self.gi), ptr(self.mod.weight), C.byref(self.y.G), None, ptr(self.mod.gradWeight),
+                   None if fused_bias else ptr(self.mod.gradBias), E.gscale)
+        E.param_done(self.mod)
+
+    def acc_units(self):
+        return [((_keys(self.y.G, self.inp.buf), _keys(self.mod.gradWeight, self.mod.gradBias)), self.bwd_param)]
 
 
 class ApplyOp(Op):
@@ -578,6 +611,26 @@ class ApplyOp(Op):
         self.bwd_combine(E)
         self.bwd_bn(E)
 
+    def bwd_input(self, E):
+        self.bwd_combine(E)
+        self.bwd_bn(E, params=False)
+
+    def param_job(self, E, job):
+        """fill the mg_bn_param_job of this layer (mg_bn_param_grad): exactly what bwd_bn adds to the parameter gradients, from the
+        sums and statistics the update phase left behind"""
+        bn = self.bn
+        job.sums, job.C = _k(self.dsums), self.out.C
+        job.gamma, job.dgamma, job.dbeta, job.conv_dbias = _k(bn.weight), _k(bn.gradWeight), _k(bn.gradBias), _k(self.conv.mod.gradBias)
+        if self.frozen:
+            job.frozen, job.count, job.gscale = 1, 0, E.gscale
+            job.running_mean, job.running_var, job.eps = _k(bn.running_mean), _k(bn.running_var), bn.eps
+            job.save_mean = job.save_invstd = None
+        else:
+            job.frozen, job.count, job.gscale = 0, self.count * max(1, E.bn_sync), E.gscale / max(1, E.bn_sync)
+            job.save_mean, job.save_invstd = _k(self.mean), _k(self.invstd)
+            job.running_mean = job.running_var = None
+            job.eps = 0.0
+
     def bwd_combine(self, E):
         if self.pc is not None:
             self.pc.run()
@@ -586,9 +639,12 @@ class ApplyOp(Op):
         else:
             self.comb.run()
 
-    def bwd_bn(self, E, synced=False):
+    def bwd_bn(self, E, synced=False, params=True):
+        """params = False (updateGradInput): G alone, no parameter gradient; the sums stay for param_job"""
         bn = self.bn
         if bn is not None and self.frozen:
+            if not params:   # the combine already wrote G
+                return
             # the sums are this rank's own: every rank adds its full share of dgamma / dbeta / gradBias, the gradient all-reduce
             # sums them like any other parameter gradient
             E.ctx.call("mg_bn_backward_frozen", ptr(self.dsums), self.out.C, ptr(bn.weight), ptr(bn.running_mean), ptr(bn.running_var),
@@ -597,12 +653,14 @@ class ApplyOp(Op):
         elif bn is not None:
             if E.bn_sync and not synced:
                 E.ctx.call("mg_allreduce_inline", ptr(self.dsums), self.dsums.numel(), 2)
+            pg = ptr if params else (lambda t: None)
             E.ctx.call("mg_bn_backward", C.byref(self.yraw), C.byref(self.dg), C.byref(self.gg), ptr(self.dsums), self.count * max(1, E.bn_sync),
-                       ptr(bn.weight), ptr(self.mean), ptr(self.invstd), ptr(bn.gradWeight), ptr(bn.gradBias),
+                       ptr(bn.weight), ptr(self.mean), ptr(self.invstd), pg(bn.gradWeight), pg(bn.gradBias),
                        # sync-BN: the sums are already global, every rank adds 1/N of dgamma / dbeta / the conv's gradBias
                        # (all derived from the sums) before the gradient all-reduce
-                       E.gscale / max(1, E.bn_sync), ptr(self.coef), ptr(self.conv.mod.gradBias))
-            E.param_done(bn)
+                       E.gscale / max(1, E.bn_sync), ptr(self.coef), pg(self.conv.mod.gradBias))
+            if params:
+                E.param_done(bn)
 
 
 class PoolOp(Op):
