@@ -82,8 +82,8 @@ class Engine:
         self._tuned_fwd = self._tuned_bwd = False
         # per-scale chains of a stage on separate CUDA streams (sched.py); MGCONV_LANES=1 runs the serial plan
         self.n_lanes = max(1, min(4, int(os.environ.get("MGCONV_LANES", "3"))))
-        self._sched_fwd = self._sched_bwd = self._sched_upd = self._sched_acc = None
-        self._acc_units = None
+        self._units = {}    # pass -> its sched.Units in execution order (ops.Op.forward_unit / backward_units), built once per plan
+        self._scheds = {}   # (pass, n_lanes) -> its lane schedule
         # split backward (updateGradInput / accGradParameters): forwards run so far, and the forward the last update_grad_input
         # differentiated -- acc_grad_parameters reads what that call left in the plan's buffers
         self.generation = 0
@@ -111,6 +111,7 @@ class Engine:
         ops.fuse_stem_pool3(b.ops, self)
         for o in b.ops:
             o.setup_fwd(self)
+        self._units["forward"] = [o.forward_unit() for o in b.ops]
         self._bwd_ready = False
 
     def _wrap_outputs(self, out, b):
@@ -175,18 +176,12 @@ class Engine:
         # cross-replica BatchNorm issues NCCL calls from inside the chains: those must stay on one stream
         return self.n_lanes > 1 and not self.bn_sync
 
-    def invalidate_schedules(self):
-        """buffer addresses the schedules were derived from changed (parameters re-homed by getParameters())"""
-        self._sched_fwd = self._sched_bwd = self._sched_upd = self._sched_acc = None
-        self._acc_units = None
-
     def _bind_stream(self):
         self.ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
 
     # ---- execution ------------------------------------------------------------------------
     def pack_weights(self):
         """fp32 master weights -> bf16 operand images of every convolution, one launch for the whole plan"""
-        import ctypes as C
         jobs = [j for o in self.conv_ops for j in o.pack_jobs()]
         if not jobs:
             return
@@ -218,16 +213,27 @@ class Engine:
                 o.tune_fwd(self)
             self._report_tuning("algo_fwd")
         self.zero_sums("fwd")
-        if self._use_lanes():
-            if self._sched_fwd is None:
-                self._sched_fwd = sched.Schedule(self.plan.ops, lambda o: o.io_fwd(), lambda o: o.fwd, self.n_lanes, 0)
-            self._sched_fwd.run(self)
-        elif self.bn_sync and training:
-            self._run_sync_bn(self.plan.ops, fwd=True)
-        else:
-            for o in self.plan.ops:
-                o.fwd(self)
+        self._run("forward")
         return self._results(self.out_struct)
+
+    def _run(self, name):
+        """run pass `name` ("forward", "backward", "update" or "acc") from its units: on the lanes, else serially, under
+        -bnSync with one all-reduce of the BatchNorm sums per run of consecutive ApplyOps"""
+        units, params = self._units[name], name != "update"
+        if self._use_lanes():
+            s = self._scheds.get((name, self.n_lanes))
+            if s is None:
+                # weight gradients (nothing but the optimiser waits for them) fill a background lane beside the chains of
+                # backward; in accGradParameters they are all there is, and spread over the lanes by size
+                bg = self.n_lanes if name == "backward" and self.n_lanes < 4 else None
+                base = 0 if name == "forward" else len(self.plan.ops) + 16   # backward event ids follow the forward's
+                s = self._scheds[name, self.n_lanes] = sched.Schedule(units, lambda u: u.io, lambda u: u.run, self.n_lanes, base, bg)
+            s.run(self, params)
+        elif self.bn_sync:
+            self._run_sync_bn(units, name == "forward", params)
+        else:
+            for u in units:
+                u.run(self, params)
 
     # ---- cross-replica BatchNorm: one all-reduce per STAGE ----------------------------------------------------------
     # The plan lists a stage as [conv of every scale ..., apply of every scale ...] and the statistics of consecutive layers
@@ -245,19 +251,19 @@ class Engine:
         self.ctx.call("mg_allreduce_inline", C.c_void_p(lo), (hi - lo) // 8, 2)
         return True
 
-    def _run_sync_bn(self, oplist, fwd, params=True):
-        """params = False: the backward of update_grad_input (no parameter gradients)"""
-        i, n = 0, len(oplist)
+    def _run_sync_bn(self, units, fwd, params):
+        """params = False: the backward of update_grad_input (no parameter gradients).  An evaluate() forward all-reduces
+        nothing: every BatchNorm is frozen."""
+        i, n = 0, len(units)
         while i < n:
-            o = oplist[i]
-            if not isinstance(o, ops.ApplyOp):
-                (o.fwd if fwd else o.bwd if params else o.bwd_input)(self)
+            if not isinstance(units[i].op, ops.ApplyOp):
+                units[i].run(self, params)
                 i += 1
                 continue
             j = i
-            while j < n and isinstance(oplist[j], ops.ApplyOp):
+            while j < n and isinstance(units[j].op, ops.ApplyOp):
                 j += 1
-            run = oplist[i:j]
+            run = [u.op for u in units[i:j]]
             if fwd:
                 synced = self._allreduce_sums([a.conv.sums for a in run if a.bn is not None and not a.frozen])
                 for a in run:
@@ -278,6 +284,9 @@ class Engine:
     def _setup_bwd(self):
         for o in reversed(self.plan.ops):
             o.setup_bwd(self)
+        units = [u for o in reversed(self.plan.ops) for u in o.backward_units()]
+        for name in ("backward", "update", "acc"):
+            self._units[name] = [u for u in units if name in u.passes]
         self._bwd_ready = True
 
     def _begin_backward(self, gradOutput):
@@ -304,25 +313,7 @@ class Engine:
         self.gscale = float(scale)
         self._begin_backward(gradOutput)
         self.grad_input_generation = None   # the buffers now hold this backward's gradient
-        if self._use_lanes():
-            if self._sched_bwd is None:
-                # a convolution's backward is two units: dgrad (the next stage waits for it) on the lane of its scale,
-                # wgrad (only the optimiser waits for it) on a background lane that fills whatever the chains leave idle
-                units = []
-                bg = self.n_lanes if (self.n_lanes < 4 and os.environ.get("MGCONV_WGRAD_LANE", "1") != "0") else None
-                for o in reversed(self.plan.ops):
-                    if isinstance(o, ops.ConvOp):
-                        units += [sched.Unit(io, run, o.size(), lane) for io, run, lane in o.bwd_units()]
-                    else:
-                        units.append(sched.Unit(o.io_bwd(), o.bwd, o.size()))
-                base = len(self.plan.ops) + 16
-                self._sched_bwd = sched.Schedule(units, lambda u: u.io, lambda u: u.run, self.n_lanes, base, background_lane=bg)
-            self._sched_bwd.run(self)
-        elif self.bn_sync:
-            self._run_sync_bn(list(reversed(self.plan.ops)), fwd=False)
-        else:
-            for o in reversed(self.plan.ops):
-                o.bwd(self)
+        self._run("backward")
         return self._grad_input()
 
     # ---- backward in the two phases of the nn protocol --------------------------------------------------------------
@@ -333,17 +324,8 @@ class Engine:
     # as in backward(), so the pair leaves backward's bits.
     def update_grad_input(self, gradOutput):
         self._begin_backward(gradOutput)
-        if self._use_lanes():
-            if self._sched_upd is None:
-                units = [sched.Unit(o.io_bwd_input(), o.bwd_input, o.size()) for o in reversed(self.plan.ops)]
-                self._sched_upd = sched.Schedule(units, lambda u: u.io, lambda u: u.run, self.n_lanes, len(self.plan.ops) + 16)
-            self._sched_upd.run(self)
-        elif self.bn_sync:
-            # the data gradient needs the global (sum d, sum d*y): the all-reduce of the sums belongs to this phase
-            self._run_sync_bn(list(reversed(self.plan.ops)), fwd=False, params=False)
-        else:
-            for o in reversed(self.plan.ops):
-                o.bwd_input(self)
+        # under -bnSync the data gradient needs the global (sum d, sum d*y): the all-reduce of the sums belongs to this phase
+        self._run("update")
         self.grad_input_generation = self.generation
         return self._grad_input()
 
@@ -362,13 +344,5 @@ class Engine:
             self.ctx.call("mg_bn_param_grad", n, self._bn_jobs)
             for o in self.bn_ops:
                 self.param_done(o.bn)
-        if self._acc_units is None:
-            self._acc_units = [sched.Unit(io, run, o.size()) for o in reversed(self.plan.ops) for io, run in o.acc_units()]
-        if self._use_lanes():
-            # the schedule starts behind everything on lane 0 (the update phase joined its lanes there, then the BatchNorm launch)
-            if self._sched_acc is None:
-                self._sched_acc = sched.Schedule(self._acc_units, lambda u: u.io, lambda u: u.run, self.n_lanes, len(self.plan.ops) + 16)
-            self._sched_acc.run(self)
-        else:
-            for u in self._acc_units:
-                u.run(self)
+        # a lane schedule starts behind everything on lane 0 (the update phase joined its lanes there, then the BatchNorm launch)
+        self._run("acc")

@@ -12,7 +12,12 @@ import os
 import torch
 
 from . import ffi
-from .ffi import mg_grid, mg_conv_desc, mg_grad_src, mg_bn_fused, mg_bn_param_job, mg_dropout, ptr, MG_SEG_SAME, MG_SEG_POOL, MG_SEG_UP, MG_SRC_POOL3, MG_MAX_SRC
+from .ffi import mg_grid, mg_conv_desc, mg_grad_src, mg_bn_fused, mg_dropout, ptr, MG_SEG_SAME, MG_SEG_POOL, MG_SEG_UP, MG_SRC_POOL3, MG_MAX_SRC
+from .sched import Unit
+
+# the passes of the engine: forward, backward, and backward in the two halves of the nn protocol -- "update"
+# (updateGradInput: data gradients, no parameter gradient) and "acc" (accGradParameters: the parameter gradients)
+BWD = ("backward", "update")
 
 
 def cpad(c):
@@ -139,21 +144,31 @@ def plan_companion_grad(E, x, p):
 
 
 class Op:
+    """Device buffers (reads, writes) of a unit are what the lane scheduler (sched.py) orders across streams; None = unknown:
+    the unit then runs on lane 0 behind a full join.  The caller's tensors (InputOp.src, grad_out), bound anew on every call
+    and touched by no other unit, are not listed."""
     def setup_fwd(self, E): pass
     def setup_bwd(self, E): pass
     def fwd(self, E): pass
-    def bwd(self, E): pass
-    # device buffers (reads, writes) of fwd() / bwd(): what the lane scheduler (sched.py) orders across streams.
-    # None = unknown: the op then runs on lane 0 behind a full join.
     def io_fwd(self): return None
-    def io_bwd(self): return None
     def size(self): return getattr(getattr(self, "out", None), "H", 0)
-    # bwd() in the two phases of the nn protocol (Engine.update_grad_input / acc_grad_parameters): bwd_input computes the
-    # gradients of the data and writes no parameter gradient; acc_units are the parameter-gradient work as (io, run) pairs.
-    # BatchNorm layers take part through ApplyOp.param_job (one batched launch of the engine) instead.
-    def bwd_input(self, E): self.bwd(E)
-    def io_bwd_input(self): return self.io_bwd()
-    def acc_units(self): return []
+
+    def forward_unit(self):
+        return Unit(self, self.io_fwd(), lambda E, params: self.fwd(E), ("forward",))
+
+    def backward_units(self):
+        """the op's work in the backward passes, in execution order, built once after setup_bwd.  run(E, params): params =
+        False in updateGradInput, which writes no parameter gradient.  BatchNorm layers add theirs in accGradParameters
+        through ApplyOp.param_job (one batched launch of the engine) instead of a unit.  Every op has a unit in backward and
+        updateGradInput, if only this empty one: the lane schedules number their events by unit."""
+        return [Unit(self, ([], []), lambda E, params: None, BWD)]
+
+
+def _combine_units(op, comb):
+    """the backward of an op whose gradient is a Combine (or nothing, comb = None)"""
+    if comb is None:
+        return Op.backward_units(op)
+    return [Unit(op, comb.io(), lambda E, params: comb.run(), BWD)]
 
 
 def _merge(*ios):
@@ -177,12 +192,7 @@ class InputOp(Op):
         self.g = self.out.grid()
 
     def io_fwd(self):
-        return _keys(self.src), _keys(self.out.buf)
-
-    def io_bwd(self):
-        if self.comb is None:
-            return [], []
-        return _merge(self.comb.io(), ([], _keys(self.grad_nchw)))
+        return [], _keys(self.out.buf)
 
     def fwd(self, E):
         E.ctx.call("mg_import_nchw", ptr(self.src), C.byref(self.g))
@@ -193,10 +203,14 @@ class InputOp(Op):
             self.grad_nchw = torch.empty((self.out.N, self.out.C, self.out.H, self.out.W), dtype=torch.float32, device=E.device)
             self.dg = self.comb.grid()
 
-    def bwd(self, E):
-        if self.comb is not None:
-            self.comb.run()
-            E.ctx.call("mg_export_nchw", C.byref(self.dg), ptr(self.grad_nchw))
+    def backward_units(self):
+        if self.comb is None:
+            return super().backward_units()
+        return [Unit(self, _merge(self.comb.io(), ([], _keys(self.grad_nchw))), self.backward, BWD)]
+
+    def backward(self, E, params):
+        self.comb.run()
+        E.ctx.call("mg_export_nchw", C.byref(self.dg), ptr(self.grad_nchw))
 
 
 class AvgPoolOp(Op):
@@ -215,11 +229,6 @@ class AvgPoolOp(Op):
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.out.buf)
 
-    def io_bwd(self):
-        if self.comb is None:
-            return [], []
-        return _merge(self.comb.io(), (_keys(self.comb.buf), _keys(self.din)))
-
     def fwd(self, E):
         E.ctx.call("mg_avgpool_forward", C.byref(self.gi), self.r, C.byref(self.go))
 
@@ -231,10 +240,14 @@ class AvgPoolOp(Op):
             self.dg_out, self.dg_in = self.comb.grid(), t.grid(self.din)
             t.srcs.append(Src(self.din, t.H, t.W, t.C, t.Cp, 0, MG_SEG_SAME))
 
-    def bwd(self, E):
-        if self.comb is not None:
-            self.comb.run()
-            E.ctx.call("mg_avgpool_backward", C.byref(self.dg_out), self.r, C.byref(self.dg_in))
+    def backward_units(self):
+        if self.comb is None:
+            return super().backward_units()
+        return [Unit(self, _merge(self.comb.io(), (_keys(self.comb.buf), _keys(self.din))), self.backward, BWD)]
+
+    def backward(self, E, params):
+        self.comb.run()
+        E.ctx.call("mg_avgpool_backward", C.byref(self.dg_out), self.r, C.byref(self.dg_in))
 
 
 def _stats(conv):
@@ -298,12 +311,6 @@ class ConvOp(Op):
         self.Ccat = sum(t.C for t, _ in self.segs)
         self.CcatP = sum(t.Cp for t, _ in self.segs)
 
-    def pack(self, E):
-        if self.wpack is not None:
-            E.ctx.call("mg_conv_pack_weights", C.byref(self.desc), ptr(self.mod.weight), ptr(self.wpack), 0)
-        if self.wpack_t is not None:
-            E.ctx.call("mg_conv_pack_weights", C.byref(self.desc), ptr(self.mod.weight), ptr(self.wpack_t), 1)
-
     def pack_jobs(self):
         """(desc, weight, packed image, transposed) of every operand image this convolution needs"""
         jobs = []
@@ -352,12 +359,6 @@ class ConvOp(Op):
     def io_fwd(self):
         return _keys(*[t.buf for t, _ in self.segs]), _keys(self.y.buf, self.sums, self.col)
 
-    def io_bwd(self):
-        io = self.ycomb.io() if self.ycomb is not None else None
-        r = _keys(self.y.G, self.col, *[t.buf for t, _ in self.segs])
-        w = _keys(self.mod.gradWeight, self.mod.gradBias, self.dcat)
-        return _merge(io, (r, w))
-
     def fwd(self, E):
         if self.col is not None:
             E.ctx.call("mg_im2col", C.byref(self.in_g), self.k, self.stride, self.pad, C.byref(self.col_g))
@@ -382,45 +383,27 @@ class ConvOp(Op):
             if nb:
                 self.wpack_t = E.alloc((nb,), torch.uint8)
 
-    def bwd_data(self, E):
-        """gradient of y from its consumers (plain convs), then dgrad: the part the rest of backward waits for"""
+    def backward_units(self):
+        """dgrad, which the rest of backward waits for, and wgrad, which only the optimiser (and the gradient all-reduce) waits
+        for: the lane schedule of backward runs it on a background lane"""
+        io_d = _merge(self.ycomb.io() if self.ycomb is not None else None,
+                      (_keys(self.y.G), _keys(self.dcat)) if self.needs_dgrad else ([], []))
+        io_w = (_keys(self.y.G, self.col, *[t.buf for t, _ in self.segs]), _keys(self.mod.gradWeight, self.mod.gradBias))
+        return [Unit(self, io_d, self.dgrad, BWD), Unit(self, io_w, self.wgrad, ("backward", "acc"), "background")]
+
+    def dgrad(self, E, params):
+        """gradient of y from its consumers (plain convs), then the gradient of the input"""
         if self.ycomb is not None:
             self.ycomb.run()
         if self.needs_dgrad:
             E.ctx.call("mg_conv_backward_data", C.byref(self.desc), ptr(self.mod.weight), ptr(self.wpack_t),
                        C.byref(self.y.G), C.byref(self.dcat_g))
 
-    def bwd_weight(self, E):
-        """accGradParameters: nothing but the optimiser (and the gradient all-reduce) waits for this"""
+    def wgrad(self, E, params):
         fused_bias = self.apply is not None and self.apply.bn is not None   # done by mg_bn_backward (from the BatchNorm sums)
         E.ctx.call("mg_conv_backward_weight", C.byref(self.desc), C.byref(self.y.G), ptr(self.mod.gradWeight),
                    None if fused_bias else ptr(self.mod.gradBias), E.gscale)
         E.param_done(self.mod)
-
-    def bwd(self, E):
-        self.bwd_data(E)
-        self.bwd_weight(E)
-
-    def bwd_input(self, E):
-        self.bwd_data(E)
-
-    def io_bwd_input(self):
-        return self.bwd_units()[0][0]
-
-    def acc_units(self):
-        io_w, run, _ = self.bwd_units()[1]
-        return [(io_w, run)]
-
-    def bwd_units(self):
-        """the two independently schedulable halves of bwd() for the lane scheduler: (io, run, fixed lane or None)"""
-        io_d = _merge(self.ycomb.io() if self.ycomb is not None else None,
-                      (_keys(self.y.G), _keys(self.dcat)) if self.needs_dgrad else ([], []))
-        io_w = (_keys(self.y.G, self.col, *[t.buf for t, _ in self.segs]), _keys(self.mod.gradWeight, self.mod.gradBias))
-        if self.needs_dgrad and os.environ.get("MGCONV_WGRAD_AFTER_DGRAD", "0") != "0":
-            # (experiment) start the weight gradient only when the layer's dgrad has finished: two tensor-bound kernels then do not
-            # share the SMs, and the weight gradient overlaps the HBM-bound passes of the next layer instead
-            io_w = (io_w[0] + _keys(self.dcat), io_w[1])
-        return [(io_d, self.bwd_data, None), (io_w, self.bwd_weight, "background")]
 
 
 class UpConvOp(Op):
@@ -446,9 +429,6 @@ class UpConvOp(Op):
         if self.want_stats:
             self.sums = E.alloc_sums(2 * self.Cout, "fwd")
 
-    def pack(self, E):
-        pass
-
     def pack_jobs(self):
         return []
 
@@ -457,10 +437,6 @@ class UpConvOp(Op):
 
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.y.buf, self.sums)
-
-    def io_bwd(self):
-        io = self.ycomb.io() if self.ycomb is not None else None
-        return _merge(io, (_keys(self.y.G, self.inp.buf), _keys(self.mod.gradWeight, self.mod.gradBias, self.dx)))
 
     def fwd(self, E):
         E.ctx.call("mg_upconv2x2_forward", C.byref(self.gi), ptr(self.mod.weight), ptr(self.mod.bias), C.byref(self.yg), _stats(self))
@@ -475,31 +451,25 @@ class UpConvOp(Op):
             self.dxg = self.inp.grid(self.dx)
             self.inp.srcs.append(Src(self.dx, self.inp.H, self.inp.W, self.inp.C, self.inp.Cp, 0, MG_SEG_SAME))
 
-    def bwd(self, E):
+    def backward_units(self):
+        """backward makes one mg_upconv2x2_backward call for dx, dw and dbias (two would launch its shuffle kernel twice);
+        updateGradInput makes it for dx alone, accGradParameters for dw and dbias alone"""
+        r, w = _keys(self.y.G, self.inp.buf), _keys(self.mod.gradWeight, self.mod.gradBias)
+        io = _merge(self.ycomb.io() if self.ycomb is not None else None, (r, w + _keys(self.dx)))
+        return [Unit(self, io, self.backward, BWD), Unit(self, (r, w), lambda E, params: self._call(E, False, True), ("acc",))]
+
+    def backward(self, E, params):
         if self.ycomb is not None:
             self.ycomb.run()
-        fused_bias = self.apply is not None and self.apply.bn is not None
-        E.ctx.call("mg_upconv2x2_backward", C.byref(self.gi), ptr(self.mod.weight), C.byref(self.y.G),
-                   C.byref(self.dxg) if self.dx is not None else None, ptr(self.mod.gradWeight),
-                   None if fused_bias else ptr(self.mod.gradBias), E.gscale)
-        E.param_done(self.mod)
+        if params or self.dx is not None:
+            self._call(E, self.dx is not None, params)
 
-    def bwd_input(self, E):
-        """the dx half of mg_upconv2x2_backward (dw, dbias NULL)"""
-        if self.ycomb is not None:
-            self.ycomb.run()
-        if self.dx is not None:
-            E.ctx.call("mg_upconv2x2_backward", C.byref(self.gi), ptr(self.mod.weight), C.byref(self.y.G), C.byref(self.dxg), None, None, E.gscale)
-
-    def bwd_param(self, E):
-        """the dw / dbias half (dx NULL)"""
-        fused_bias = self.apply is not None and self.apply.bn is not None
-        E.ctx.call("mg_upconv2x2_backward", C.byref(self.gi), ptr(self.mod.weight), C.byref(self.y.G), None, ptr(self.mod.gradWeight),
-                   None if fused_bias else ptr(self.mod.gradBias), E.gscale)
-        E.param_done(self.mod)
-
-    def acc_units(self):
-        return [((_keys(self.y.G, self.inp.buf), _keys(self.mod.gradWeight, self.mod.gradBias)), self.bwd_param)]
+    def _call(self, E, dx, params):
+        fused_bias = self.apply is not None and self.apply.bn is not None   # done by mg_bn_backward (from the BatchNorm sums)
+        E.ctx.call("mg_upconv2x2_backward", C.byref(self.gi), ptr(self.mod.weight), C.byref(self.y.G), C.byref(self.dxg) if dx else None,
+                   ptr(self.mod.gradWeight) if params else None, None if fused_bias or not params else ptr(self.mod.gradBias), E.gscale)
+        if params:
+            E.param_done(self.mod)
 
 
 class ApplyOp(Op):
@@ -562,14 +532,6 @@ class ApplyOp(Op):
             w += _keys(self.scale, self.shift, self.mean, self.invstd)
         return r, w
 
-    def io_bwd(self):
-        io = _merge(self.pc.io() if self.pc is not None else None, self.comb.io())
-        if self.bn is not None:
-            bn = self.bn
-            io = _merge(io, (_keys(self.conv.y.buf, self.comb.buf, self.dsums, self.mean, self.invstd),
-                             _keys(self.G, bn.gradWeight, bn.gradBias, self.conv.mod.gradBias)))
-        return io
-
     def fwd(self, E, synced=False):
         """synced: the engine has already all-reduced this layer's statistics together with those of the other scales of the stage"""
         bn = self.bn
@@ -607,17 +569,22 @@ class ApplyOp(Op):
         else:
             y.G = t.grid(D)
 
-    def bwd(self, E):
-        self.bwd_combine(E)
-        self.bwd_bn(E)
+    def backward_units(self):
+        """one unit: the engine's -bnSync path runs the two halves, bwd_combine and bwd_bn, itself"""
+        io = _merge(self.pc.io() if self.pc is not None else None, self.comb.io())
+        if self.bn is not None:
+            bn = self.bn
+            io = _merge(io, (_keys(self.conv.y.buf, self.comb.buf, self.dsums, self.mean, self.invstd),
+                             _keys(self.G, bn.gradWeight, bn.gradBias, self.conv.mod.gradBias)))
+        return [Unit(self, io, self.backward, BWD)]
 
-    def bwd_input(self, E):
+    def backward(self, E, params):
         self.bwd_combine(E)
-        self.bwd_bn(E, params=False)
+        self.bwd_bn(E, params=params)
 
     def param_job(self, E, job):
         """fill the mg_bn_param_job of this layer (mg_bn_param_grad): exactly what bwd_bn adds to the parameter gradients, from the
-        sums and statistics the update phase left behind"""
+        sums and statistics updateGradInput left behind"""
         bn = self.bn
         job.sums, job.C = _k(self.dsums), self.out.C
         job.gamma, job.dgamma, job.dbeta, job.conv_dbias = _k(bn.weight), _k(bn.gradWeight), _k(bn.gradBias), _k(self.conv.mod.gradBias)
@@ -678,18 +645,14 @@ class PoolOp(Op):
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.out.buf)
 
-    def io_bwd(self):
-        return self.pc.io() if self.pc is not None else ([], [])
-
     def fwd(self, E):
         E.ctx.call("mg_pool_forward", C.byref(self.gi), C.byref(self.go), 0, None)
 
     def setup_bwd(self, E):
         self.pc = plan_companion_grad(E, self.inp, self.out)
 
-    def bwd(self, E):
-        if self.pc is not None:
-            self.pc.run()
+    def backward_units(self):
+        return _combine_units(self, self.pc)
 
 
 class Pool3Op(Op):
@@ -711,9 +674,6 @@ class Pool3Op(Op):
             return [], []
         return _keys(self.inp.buf), _keys(self.out.buf, self.code)
 
-    def io_bwd(self):
-        return self.comb.io() if self.comb is not None else ([], [])
-
     def fwd(self, E):
         if not self.fused:
             E.ctx.call("mg_pool3s2_forward", C.byref(self.gi), C.byref(self.go), ptr(self.code))
@@ -725,9 +685,8 @@ class Pool3Op(Op):
             self.comb = Combine(E, t)
             self.inp.srcs.append(Src(self.comb.buf, t.H, t.W, t.C, t.Cp, 0, MG_SRC_POOL3, aux=self.code))
 
-    def bwd(self, E):
-        if self.comb is not None:
-            self.comb.run()
+    def backward_units(self):
+        return _combine_units(self, self.comb)
 
 
 def _tensor_refs(op):
@@ -777,9 +736,6 @@ class CatOp(Op):
     def io_fwd(self):
         return _keys(*[p.buf for p in self.parts]), _keys(self.out.buf)
 
-    def io_bwd(self):
-        return self.comb.io() if self.comb is not None else ([], [])
-
     def fwd(self, E):
         off = 0
         for p, g in zip(self.parts, self.gp):
@@ -797,9 +753,8 @@ class CatOp(Op):
                     p.srcs.append(Src(self.comb.buf, t.H, t.W, t.C, t.Cp, off, MG_SEG_SAME))
                 off += p.C
 
-    def bwd(self, E):
-        if self.comb is not None:
-            self.comb.run()
+    def backward_units(self):
+        return _combine_units(self, self.comb)
 
 
 class DropStepOp(Op):
@@ -811,9 +766,6 @@ class DropStepOp(Op):
 
     def io_fwd(self):
         return [], _keys(self.step)
-
-    def io_bwd(self):
-        return [], []
 
     def fwd(self, E):
         E.ctx.call("mg_dropout_advance", ptr(self.step))
@@ -840,11 +792,6 @@ class DropOp(Op):
     def io_fwd(self):
         return _keys(self.step_op.step, *[t.buf for t, _ in self.segs]), _keys(self.out.buf)
 
-    def io_bwd(self):
-        if self.comb is None:
-            return [], []
-        return _merge(self.comb.io(), (_keys(self.step_op.step, self.comb.buf), _keys(self.comb.buf)))
-
     def fwd(self, E):
         E.ctx.call("mg_dropout_forward", C.byref(self.dp), len(self.segs), self.sg, self.sm, C.byref(self.go))
 
@@ -860,10 +807,14 @@ class DropOp(Op):
                     p.srcs.append(Src(self.comb.buf, t.H, t.W, t.C, t.Cp, off, m))
                 off += p.C
 
-    def bwd(self, E):
-        if self.comb is not None:
-            self.comb.run()
-            E.ctx.call("mg_dropout_backward", C.byref(self.dp), C.byref(self.dg))
+    def backward_units(self):
+        if self.comb is None:
+            return super().backward_units()
+        return [Unit(self, _merge(self.comb.io(), (_keys(self.step_op.step, self.comb.buf), _keys(self.comb.buf))), self.backward, BWD)]
+
+    def backward(self, E, params):
+        self.comb.run()
+        E.ctx.call("mg_dropout_backward", C.byref(self.dp), C.byref(self.dg))
 
 
 class GlobalAvgOp(Op):
@@ -880,9 +831,6 @@ class GlobalAvgOp(Op):
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.out.buf)
 
-    def io_bwd(self):
-        return _merge(self.comb.io(), (_keys(self.comb.buf), _keys(self.din)))
-
     def fwd(self, E):
         E.ctx.call("mg_global_avgpool_forward", C.byref(self.gi), C.byref(self.go))
 
@@ -892,7 +840,10 @@ class GlobalAvgOp(Op):
         self.dg_out, self.dg_in = self.comb.grid(), self.inp.grid(self.din)
         self.inp.srcs.append(Src(self.din, self.inp.H, self.inp.W, self.inp.C, self.inp.Cp, 0, MG_SEG_SAME))
 
-    def bwd(self, E):
+    def backward_units(self):
+        return [Unit(self, _merge(self.comb.io(), (_keys(self.comb.buf), _keys(self.din))), self.backward, BWD)]
+
+    def backward(self, E, params):
         self.comb.run()
         E.ctx.call("mg_global_avgpool_backward", C.byref(self.dg_out), C.byref(self.dg_in))
 
@@ -911,9 +862,6 @@ class LogSoftMaxOp(Op):
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.result)
 
-    def io_bwd(self):
-        return _keys(self.result, self.grad_out), _keys(self.dl)
-
     def fwd(self, E):
         E.ctx.call("mg_logsoftmax_forward", C.byref(self.gi), ptr(self.result))
 
@@ -923,7 +871,10 @@ class LogSoftMaxOp(Op):
         self.inp.srcs.append(Src(self.dl, 1, 1, self.inp.C, self.inp.Cp, 0, MG_SEG_SAME))
         self.grad_out = None
 
-    def bwd(self, E):
+    def backward_units(self):
+        return [Unit(self, (_keys(self.result), _keys(self.dl)), self.backward, BWD)]
+
+    def backward(self, E, params):
         E.ctx.call("mg_logsoftmax_backward", ptr(self.result), ptr(self.grad_out), C.byref(self.dlg))
 
 
@@ -942,9 +893,6 @@ class SigmoidOp(Op):
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.result)
 
-    def io_bwd(self):
-        return _keys(self.result, self.grad_out), _keys(self.dx)
-
     def fwd(self, E):
         E.ctx.call("mg_sigmoid_forward", C.byref(self.gi), ptr(self.result))
 
@@ -955,7 +903,10 @@ class SigmoidOp(Op):
         t.srcs.append(Src(self.dx, t.H, t.W, t.C, t.Cp, 0, MG_SEG_SAME))
         self.grad_out = None
 
-    def bwd(self, E):
+    def backward_units(self):
+        return [Unit(self, (_keys(self.result), _keys(self.dx)), self.backward, BWD)]
+
+    def backward(self, E, params):
         E.ctx.call("mg_sigmoid_backward", ptr(self.result), ptr(self.grad_out), C.byref(self.dxg))
 
 
@@ -977,9 +928,6 @@ class ExportOp(Op):
     def io_fwd(self):
         return _keys(self.inp.buf), _keys(self.result)
 
-    def io_bwd(self):
-        return _keys(self.grad_out), _keys(self.dx)
-
     def fwd(self, E):
         E.ctx.call("mg_export_nchw", C.byref(self.gi), ptr(self.result))
 
@@ -990,5 +938,8 @@ class ExportOp(Op):
         t.srcs.append(Src(self.dx, t.H, t.W, t.C, t.Cp, 0, MG_SEG_SAME))
         self.grad_out = None
 
-    def bwd(self, E):
+    def backward_units(self):
+        return [Unit(self, ([], _keys(self.dx)), self.backward, BWD)]
+
+    def backward(self, E, params):
         E.ctx.call("mg_import_nchw", ptr(self.grad_out), C.byref(self.dxg))

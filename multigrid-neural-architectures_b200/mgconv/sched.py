@@ -2,9 +2,9 @@
 
 Within one mg stage the chain conv -> BatchNorm -> ReLU of every grid (models/ilsvrc/rnmg.lua:91-159) only
 meets the other grids again at the next ResampleConcat, and most of those kernels (14x14, 7x7 ... grids) are
-far too small to fill 148 SMs.  Each plan op declares the device buffers it reads and writes (ops.io_fwd /
-io_bwd); ops are assigned a lane by the spatial size they work on, and this module derives -- once per plan and
-pass -- the cross-lane event waits that keep every read-after-write, write-after-read and write-after-write
+far too small to fill 148 SMs.  Each plan op declares its work as units with the device buffers they read and
+write (ops.Op.forward_unit / backward_units); units are assigned a lane by the spatial size they work on, and this
+module derives -- once per plan and pass -- the cross-lane event waits that keep every read-after-write, write-after-read and write-after-write
 pair ordered.  Execution order on each lane is the plan order, so a single lane reproduces the serial plan.
 
 The schedule is static: (lane switch, event waits, op, event record) tuples replayed through the C ABI
@@ -14,10 +14,12 @@ ends with lane 0 waiting for all lanes, so nothing outside the pass ever sees a 
 
 
 class Unit:
-    """a schedulable piece of an op: buffers (reads, writes), callable(E), spatial size, optional fixed lane"""
+    """a schedulable piece of an op's work: buffers (reads, writes) or None, run(E, params), the engine passes it belongs
+    to, optional fixed lane ("background"); its spatial size is the op's"""
 
-    def __init__(self, io, run, size, lane=None):
-        self.io, self.run, self._size, self.lane = io, run, size, lane
+    def __init__(self, op, io, run, passes, lane=None):
+        self.op, self.io, self.run, self.passes, self.lane = op, io, run, passes, lane
+        self._size = op.size()
 
     def size(self):
         return self._size
@@ -93,7 +95,8 @@ class Schedule:
                 ctx.call("mg_ctx_event_wait", self.ev_base + 1 + self.n_ops + l)
         return 0
 
-    def run(self, E):
+    def run(self, E, *args):
+        """args: passed on to every op's run after E"""
         ctx = E.ctx
         cur = 0
         try:
@@ -107,7 +110,7 @@ class Schedule:
                         cur = lane
                     for ds in waits:
                         ctx.call("mg_ctx_event_wait", self._ev(ds))
-                run(E)
+                run(E, *args)
                 if seq in self.record:
                     ctx.call("mg_ctx_event_record", self._ev(seq))
             self._join(ctx, cur)
